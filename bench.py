@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — closed-loop RTI-MPC + RGP control steps/sec on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one closed-loop control step of EVERY vehicle on this rank: reference chunk -> RTI solve (RK4+sens,
@@ -18,8 +18,11 @@ Legs of one run (all in the same JSON line; every key says which leg it belongs 
   lemniscate_leg   N = 1 only: BASELINE configs[4], 16384 vehicles, v_peak 20 m/s (thrust limits active), >= 200 steps, p99
   shared_rgp_leg   N > 1 only: BASELINE configs[2], 65536 vehicles over the ranks, ONE shared RGP, all-reduce every step
   cpu_baseline     N = 1 only: the C oracle on the host cores (+ the numpy RGP restatement on 1 core)
+
+The library is not built here: run __graft_entry__.build() first.  bench.py writes nothing into the source tree.
 """
 import argparse
+import atexit
 import ctypes as C
 import gc
 import json
@@ -34,6 +37,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: no __pycache__ next to the package
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")   # one hardware queue per vehicle-group stream
 
 METRIC = "closed_loop_rti_mpc_rgp_control_steps_per_sec"
@@ -68,7 +72,11 @@ def parse():
     ap.add_argument("--no-extra-legs", action="store_true", help="skip the lemniscate (N=1) / shared-RGP (N>1) legs")
     ap.add_argument("--lemniscate-batch", type=int, default=16384)
     ap.add_argument("--swarm-total", type=int, default=65536, help="vehicles of the shared-RGP leg, over all ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what their last step computed to DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     a.policy = {kv.split("=")[0]: int(kv.split("=")[1]) for kv in a.solver_opts.split(",") if kv}
     return a
 
@@ -86,6 +94,29 @@ def workload_config(a, n_gpus):
             "groups_per_gpu": a.groups,
             "l2": "per-step working set (stage tiles 136 MB + factors 47 MB + RGP covariances 39 MB at the default "
                   "shape) exceeds the 126 MB L2; no explicit flush"}
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, B):
+    """Writes the arrays a caller of the timed closed loop holds after its last step (rank 0's vehicles, in order) as
+    out_dir/<name>.npy (float64): u0 [B,4] the control applied, x [B,13] the plant state after the control period,
+    x_pred [B,13] the nominal one-period prediction, x_opt [B,N+1,13] / w_opt [B,N,4] the solver iterate, and with an
+    RGP rgp_mu [*,3,M] / rgp_C [*,3,M,M] (one model per vehicle, or one shared).  Above DUMP_BYTES in all, the
+    per-vehicle arrays keep a fixed seeded sample of vehicles whose indices go to vehicle_index.npy."""
+    per_vehicle = {k for k, v in arrays.items() if v.shape[0] == B}
+    vehicle_bytes = sum(arrays[k][0].size for k in per_vehicle) * 8
+    shared_bytes = sum(v.size for k, v in arrays.items() if k not in per_vehicle) * 8
+    keep = max(1, min(B, (DUMP_BYTES - shared_bytes) // (vehicle_bytes + 8)))     # + 8: its entry in vehicle_index
+    idx = None if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        if idx is not None and k in per_vehicle:
+            v = v[idx]
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(v, dtype=np.float64))
+    if idx is not None:
+        np.save(os.path.join(out_dir, "vehicle_index.npy"), idx.astype(np.float64))
 
 
 def make_trajectories(a, first_vehicle, count, K):
@@ -147,6 +178,11 @@ def reference_arm(a):
     t0 = time.perf_counter()
     loop.run(a.steps, log=False)
     el = time.perf_counter() - t0
+    if a.dump_outputs:
+        out = {"u0": loop.uit[:, 0], "x": loop.x, "x_pred": loop.xpred_prev, "x_opt": loop.xit, "w_opt": loop.uit}
+        if gp is not None:
+            out.update(rgp_mu=loop.mu, rgp_C=loop.C)
+        dump_outputs(a.dump_outputs, out, Bs)
     val = Bs * a.steps / el
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
             "warmup": a.warmup, "ms_per_step": 1e3 * el / a.steps, "higher_is_better": True, "scaling": "weak",
@@ -175,6 +211,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "10",
                                        "-i", str(index)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)          # never outlives bench.py, also when a leg raises before stop()
         except Exception:
             self.p = None
 
@@ -310,10 +347,7 @@ def flops_per_step(N, M, n_ipm):
 def b200_arm(a):
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as graft
     rank, world, local = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
-    if rank == 0:
-        graft.build()
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device(f"cuda:{local}"))
         dist.barrier()
@@ -399,6 +433,16 @@ def b200_arm(a):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * B * a.steps / (ms_max * 1e-3)
+    if a.dump_outputs and rank == 0:
+        lps = loop.loops if grouped else [loop]
+        host = lambda ts: torch.cat(ts).cpu().numpy()
+        its = [lp.opt.get_iterate() for lp in lps]
+        out = {"u0": host([lp.u0 for lp in lps]), "x": host([lp.x for lp in lps]), "x_pred": host([lp.x_pred_prev for lp in lps]),
+               "x_opt": host([i[0] for i in its]), "w_opt": host([i[1] for i in its])}
+        if M:
+            gpes = [lp.opt.gpe for lp in lps]
+            out.update(rgp_mu=host([g.mu_tensor() for g in gpes]), rgp_C=host([g.C_tensor() for g in gpes]))
+        dump_outputs(a.dump_outputs, out, B)
 
     # ---------------- roofline leg: same steps again on ONE stream with cudaEvents around the solve kernels
     loop2 = make_loop()
