@@ -139,6 +139,18 @@ int qmpc_reset_warm_start(qmpc_handle_t h, void *stream);
 /* sum over vehicles of IPM iterations of the last solve (host value; synchronises `stream`) */
 int qmpc_iters_total(qmpc_handle_t h, long long *total, void *stream);
 
+/* acados eval_param_sens(field "ex") + get(k, "sens_x" / "sens_u") for every vehicle and every x0 component at once:
+ * derivatives of the last solve's x[k], u[k] w.r.t. x0 at the active set the handle holds (after a solve: that solve's),
+ * k < n_stages (1..N).  sens_x [B][n_stages+1][13][13] (may be NULL), sens_u [B][n_stages][4][13], row-major,
+ * column = x0 component.  NaN for vehicles whose active set is unknown.  Reads the stage tiles of the last solve:
+ * valid until the next qmpc_solve / qmpc_step on the handle.  Asynchronous.
+ * The linearisation of an RTI step does not read x0, so x0 -> (x, u) is the box-QP's solution map (piecewise affine):
+ * these are its exact derivatives on the active set, i.e. the closed loop of the LQR with the inputs flagged 1/2 pinned
+ * (their rows are 0), taken w.r.t. the 13 raw components of x0.  sens_u[:, 0] is the feedback gain K0 = du0/dx0.
+ * A solve that ended on the IPM alone (status 0) leaves the IPM's classification of the bounds; the sensitivities refer
+ * to that set.  Returns QMPC_ERR_ARG before the handle's first solve and for fp32 handles. */
+int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double *sens_x, double *sens_u, void *stream);
+
 /* ---- stateless helpers of the loop (any B) */
 /* quad_optimizer.discrete_dynamics (quad_opt.py:353-377): nominal RK4 step, optional body-frame velocity.
  * x [B][13], u [B][4] -> x_next [B][13] */

@@ -81,6 +81,7 @@ struct qmpc_solver {
     bool timing = false;              // cudaEvents around the two solve kernels (bench roofline leg only)
     std::vector<cudaEvent_t> ev;      // triples: before linearize, before ipm, after ipm
     std::vector<cudaEvent_t> ev_mid;  // between the screening and the dense kernel (one per timed solve)
+    bool solved = false;              // a solve has been queued: the stage tiles W hold data (qmpc_eval_sens_x0)
 };
 
 struct qrgp_model {
@@ -155,6 +156,8 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
     if (smem64 > 220 * 1024) return fail(QMPC_ERR_ARG, "n_nodes too large for the shared-memory plan");
     CU_TRY(cudaFuncSetAttribute(qmpc_ipm_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem64));
     CU_TRY(cudaFuncSetAttribute(qmpc_ipm_kernel<float, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
+    CU_TRY(cudaFuncSetAttribute(qmpc_sens_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     h->variant = solver_variant(h->cfg, DN_MAX_N);
     if (h->variant == 2) {
         const int smemd = dense_layout((int)N).total * 8;
@@ -334,6 +337,22 @@ static int solve_impl(qmpc_solver* h, void* stream)
     }
     LAUNCH_CHECK();
     if (e2) CU_TRY(cudaEventRecord(e2, S(stream)));
+    h->solved = true;
+    return QMPC_OK;
+}
+
+static int sens_impl(qmpc_solver* h, int n_stages, double* sens_x, double* sens_u, void* stream)
+{
+    typedef double real;
+    const int B = h->cfg.batch;
+    SensArgs<real> sa;
+    fill_sens_args(h->cfg, n_stages, sa);
+    sa.b.x0 = nullptr; sa.b.yref = nullptr; sa.b.yref_e = h->yref_e; sa.b.xit = h->xit; sa.b.uit = nullptr;
+    sa.b.W = static_cast<const real*>(h->W); sa.b.fac = static_cast<real*>(h->fac); sa.b.act = h->act;
+    sa.sens_x = sens_x; sa.sens_u = sens_u;
+    const size_t smem = (size_t)IPM_WARPS * sa.b.smem_per_warp * sizeof(real);
+    qmpc_sens_kernel<real, IPM_WARPS><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(sa);
+    LAUNCH_CHECK();
     return QMPC_OK;
 }
 
@@ -343,6 +362,17 @@ int qmpc_solve(qmpc_handle_t h, void* stream)
 {
     if (!h) return fail(QMPC_ERR_ARG, "null handle");
     return h->cfg.precision == 64 ? solve_impl<double>(h, stream) : solve_impl<float>(h, stream);
+}
+
+int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double* sens_x, double* sens_u, void* stream)
+{
+    if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    if (n_stages < 1 || n_stages > h->cfg.n_nodes) return fail(QMPC_ERR_ARG, "n_stages must be in [1, n_nodes]");
+    if (!sens_u) return fail(QMPC_ERR_ARG, "sens_u is NULL");
+    // fp32 tiles and an fp32 Riccati recursion without the solve's fp64 refinement: up to 1.4e-3 relative on a B200 (DESIGN §4)
+    if (h->cfg.precision != 64) return fail(QMPC_ERR_ARG, "sensitivities need an fp64 handle (precision 64)");
+    if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
+    return sens_impl(h, n_stages, sens_x, sens_u, stream);
 }
 
 int qmpc_get_u0(qmpc_handle_t h, double* u0, void* stream)

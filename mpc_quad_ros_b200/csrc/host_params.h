@@ -152,4 +152,15 @@ inline void fill_screen_args(const qmpc_config& c, IpmArgs<real>& a)
     a.refine_off = 0;
 }
 
+// qmpc_eval_sens_x0: weights of the solve, per-warp shared memory of the screening layout; the caller sets the pointers
+template <typename real>
+inline void fill_sens_args(const qmpc_config& c, int n_stages, SensArgs<real>& a)
+{
+    fill_ipm_args(c, a.b);
+    a.b.smem_per_warp = ipm_smem_reals(c.n_nodes, false, sizeof(real) == 8);
+    a.b.ring_off = ipm_ring_off(c.n_nodes, false);
+    a.b.refine_off = 0;
+    a.n_stages = n_stages;
+}
+
 }  // namespace qmpc

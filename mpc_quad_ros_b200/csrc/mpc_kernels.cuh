@@ -9,6 +9,8 @@
 //       Replaces acados SQP_RTI + full condensing + HPIPM (reference src/quad_opt.py:146-151,333;
 //       src/_acados_ocp.json:2082-2110).  Full step, un-shifted persistent iterate, objective at the new
 //       iterate (SURVEY.md App. A.3).
+//   qmpc_sens_kernel      : behind qmpc_eval_sens_x0, not part of a solve: derivatives of the last solve's x[k], u[k] with
+//       respect to x0 (acados eval_param_sens "ex"), one OCP per warp from the tiles and the active set the solve left.
 //
 // Per-stage tile written by K1 and streamed by K2 (HBM/L2, `real`):   W[13 rows][16 cols], row stride WR
 //   cols 0..3  = B = dPhi/du            cols 4..13 = dPhi/dx_s for s = 3..12 (q,v,r)
@@ -1051,6 +1053,65 @@ struct WarpCtx {
         }
         return cost;
     }
+
+    // Sensitivity sweep w.r.t. x0 of the pinned LQR whose factors backward_full<true>() left in `fac`: the 13 columns of
+    // dx_0 = I go through the stages with the algebra of forward<0, true> without offsets, du = -Lam^-T Lx^T dx (pinned
+    // rows 0), dx+ = A dx + B du.  Lane c < 13 carries column c in registers; tile rows, factor records and fx are
+    // broadcasts.  Stores du_k to su[k][4][13] and dx_k to sx[k][13][13] (sx may be null), lanes c < 13 writing
+    // consecutive doubles of every row.  Covers stages 0..N-1 of the context (the caller may shorten N).
+    __device__ void forward_sens(double* sx, double* su)
+    {
+        const int c = lane < NX ? lane : NX - 1;     // lanes 13..31 follow column 12 and store nothing
+        real dx[NX];
+#pragma unroll
+        for (int i = 0; i < NX; ++i) dx[i] = i == c ? real(1) : real(0);
+        if (sx && lane < NX) {
+#pragma unroll
+            for (int i = 0; i < NX; ++i) sx[i * NX + lane] = double(dx[i]);
+        }
+        sweep_begin(0, 1);
+        for (int k = 0; k < N; ++k) {
+            const real* t = tile_at(k, k);
+            const real* f = facv + (size_t)k * FAC;
+            Chol4<double> L;
+            L.load(f + 56);
+            real v[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int s_ = 0; s_ < NX; ++s_) {
+                real l0, l1, l2, l3;
+                ld2(f + s_ * 4, l0, l1); ld2(f + s_ * 4 + 2, l2, l3);
+                v[0] = fma(l0, dx[s_], v[0]); v[1] = fma(l1, dx[s_], v[1]);
+                v[2] = fma(l2, dx[s_], v[2]); v[3] = fma(l3, dx[s_], v[3]);
+            }
+            real du[4];
+            L.bsolve_neg(v, du);
+#pragma unroll
+            for (int aa = 0; aa < 4; ++aa) if (fx[k * 4 + aa] != real(0)) du[aa] = 0;
+            real xn[NX];
+#pragma unroll
+            for (int i = 0; i < NX; ++i) {
+                const real* row = t + i * WR;
+                real acc = i < 3 ? dx[i] : real(0);             // position columns of A: unit vectors, not stored
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) acc = fma(tld(row + aa), du[aa], acc);
+#pragma unroll
+                for (int s_ = 3; s_ < NX; ++s_) acc = fma(tld(row + 1 + s_), dx[s_], acc);
+                xn[i] = acc;
+            }
+            __syncwarp();                       // every lane has read the tile
+            tile_done(k, k + RING);
+            if (lane < NX) {
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) su[(k * NU + aa) * NX + lane] = double(du[aa]);
+                if (sx) {
+#pragma unroll
+                    for (int i = 0; i < NX; ++i) sx[((k + 1) * NX + i) * NX + lane] = double(xn[i]);
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < NX; ++i) dx[i] = xn[i];
+        }
+    }
 };
 
 #ifndef QMPC_IPM_MIN_WARPS
@@ -1344,6 +1405,81 @@ __global__ void __launch_bounds__(WARPS * 32, QMPC_IPM_MIN_WARPS / WARPS) qmpc_i
     if (lane < 4) a.u0[(size_t)ocp * 4 + lane] = double(c.ucur[lane]);
     if (lane == 0) { a.cost[ocp] = double(cost); a.status[ocp] = status; a.iters[ocp] = it; a.rounds[ocp] = rounds; }
     if (a.timeline && lane == 0) a.timeline[2 * ocp + 1] = global_ns();
+}
+
+// ------------------------------------------------------------------------------------------ sensitivities w.r.t. x0
+
+template <typename real>
+struct SensArgs {
+    IpmArgs<real> b;        // read: B, N, weights, W, fac (scratch between solves, rewritten here), act, xit, yref_e,
+                            // smem_per_warp / ring_off of the screening layout
+    int n_stages;           // 1..N: stages 0..n_stages-1 are swept
+    double* sens_x;         // [B][n_stages+1][13][13] or null
+    double* sens_u;         // [B][n_stages][4][13]
+};
+
+// RTI never reads x0 in K1, so x0 -> (x, u) is the box-QP's solution map: piecewise affine, and on the active set the
+// solve ended on its Jacobian is the closed loop of the LQR with those inputs pinned.  One warp per OCP: the pinned
+// factorisation of the active-set rounds (backward_full<true>), then forward_sens.  A vehicle whose active set is
+// unknown (any entry 255) gets NaN everywhere.
+// resident warps per SM the register allocation is sized for: at 16 (the solver kernel's) the fp64 factorisation spills;
+// 12 leaves it 167 registers and no spill
+constexpr int SENS_MIN_WARPS = 12;
+
+template <typename real, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_sens_kernel(SensArgs<real> s)
+{
+    QMPC_DYN_SMEM(smem_raw);
+    const IpmArgs<real>& a = s.b;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int ocp = blockIdx.x * WARPS + warp;
+    if (ocp >= a.B) return;
+    const int N = a.N, E = 4 * N, ns = s.n_stages;
+    const unsigned char* act = a.act + (size_t)ocp * E;
+    double* sx = s.sens_x ? s.sens_x + (size_t)ocp * (ns + 1) * NX * NX : nullptr;
+    double* su = s.sens_u + (size_t)ocp * ns * NU * NX;
+    int known = 1;
+    for (int e = lane; e < E; e += 32) if (act[e] > 2) known = 0;
+    if (!warp_min(known)) {
+        const double qnan = nan("");
+        if (sx) for (int i = lane; i < (ns + 1) * NX * NX; i += 32) sx[i] = qnan;
+        for (int i = lane; i < ns * NU * NX; i += 32) su[i] = qnan;
+        return;
+    }
+    // the set-up of qmpc_ipm_kernel in its screening layout (kept separate: that kernel's code is tuned); the sweeps used
+    // here read the per-warp work space, rdel, fx, fv, the tiles, `fac`, and xit / yref_e for the (unused) costate offset
+    real* sm = reinterpret_cast<real*>(smem_raw) + (size_t)warp * a.smem_per_warp;
+    WarpCtx<real> c{a};
+    c.lane = lane; c.h = lane >> 4; c.j = lane & 15; c.ocp = ocp; c.N = N; c.E = E;
+    c.hmask = 0xffffu << (lane & 16);
+    c.sidx = (c.j < 3) ? c.j : ((c.j >= 4 && c.j < 14) ? c.j - 1 : -1);
+    c.P = sm + SM_P; c.pv = sm + SM_PV; c.wv = sm + SM_WV; c.xp = sm + SM_XP; c.hv = sm + SM_HV;
+    c.Ls = sm + SM_LS; c.cs = sm + SM_CS;
+    real* v = sm + SM_VEC;
+    c.usol = c.ua = c.ucur = c.ubar = c.grad = v; c.rdel = v + 3 * E; c.cl = v + 4 * E; c.cu = v + 5 * E;
+    c.xtr = v + 6 * E;
+    c.rt = c.dR = c.ll = c.lu = c.tl = c.tu = v;
+    c.fx = c.cl; c.fv = c.cu;
+    c.hist_store = sm + a.ring_off;
+    c.ring = sm + a.ring_off + HIST_REALS<real>();
+    c.rbar = reinterpret_cast<unsigned long long*>(c.ring + WarpCtx<real>::RING * WT);
+    c.rphase = 0;
+    c.gave_up = false;
+    if (WarpCtx<real>::RING) {
+        if (lane == 0) for (int s_ = 0; s_ < WarpCtx<real>::RING; ++s_) mbar_init(c.rbar + s_, 1);
+        __syncwarp();
+    }
+    c.Wv = a.W + (size_t)ocp * N * WT;
+    c.facv = a.fac + (size_t)ocp * N * FAC;
+    c.x0 = nullptr; c.yref = nullptr; c.uit = nullptr;
+    c.yref_e = a.yref_e + (size_t)ocp * NX;
+    c.xit = a.xit + (size_t)ocp * (N + 1) * NX;
+    // homogeneous problem: pinned inputs at 0, no input gradient (the offsets only reach lg / p, never the factors)
+    for (int e = lane; e < E; e += 32) { c.fx[e] = real(act[e]); c.fv[e] = 0; c.rdel[e] = 0; }
+    __syncwarp();
+    c.template backward_full<true>();
+    c.N = ns;              // the sweep streams stages 0..ns-1 only: no tile copy is in flight when the warp exits
+    c.forward_sens(sx, su);
 }
 
 }  // namespace qmpc

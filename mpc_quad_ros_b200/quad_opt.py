@@ -68,6 +68,7 @@ class quad_optimizer:
             _capi.check(_capi.lib().qmpc_create(C.byref(cfg), C.byref(self._h)))
         self._Kx_inv = None if gpe is None else torch.as_tensor(gpe.K_x_inv, device=self.device).contiguous()
         self.yref = self.yref_N = None
+        self._numpy_io = self.batch == 1      # eval_sens answers like the last run_optimization (numpy for one vehicle)
 
     def __del__(self):
         try:
@@ -126,6 +127,7 @@ class quad_optimizer:
         if x_init is None:
             raise ValueError("x_init has to be set before running the optimization")
         single = self._single(x_init)
+        self._numpy_io = single
         x0 = self._dev(x_init, (self.batch, 13))
         lib = _capi.lib()
         t0 = time.perf_counter()
@@ -142,6 +144,21 @@ class quad_optimizer:
             c = float(cost[0].item())
             return out[0], out[1], time.perf_counter() - t0, c
         return x_opt, w_opt, time.perf_counter() - t0, cost
+
+    def eval_sens(self, n_stages=None, states=True):
+        """acados eval_param_sens(field="ex") + get(k, "sens_u" / "sens_x"): derivatives of the last solve's u[k], x[k]
+        w.r.t. x0 at the active set that solve ended on (qmpc_eval_sens_x0), for every x0 component at once.
+        n_stages (default N): stages covered, 1 gives the feedback gain sens_u[0] = du0/dx0 and sens_x[1] only.
+        returns (sens_x [n+1,13,13] or None when states=False, sens_u [n,4,13]), column = x0 component; batched: CUDA
+        tensors with a leading B.  NaN for vehicles whose active set is unknown (a failed solve).  Valid until the next
+        solve: the derivatives are taken from that solve's linearisation.  fp64 handles only (QmpcError otherwise)."""
+        n = self.n_nodes if n_stages is None else int(n_stages)
+        sx = torch.empty((self.batch, max(n, 0) + 1, 13, 13), dtype=torch.float64, device=self.device) if states else None
+        su = torch.empty((self.batch, max(n, 0), 4, 13), dtype=torch.float64, device=self.device)
+        _capi.check(_capi.lib().qmpc_eval_sens_x0(self._h, n, _capi.ptr(sx), _capi.ptr(su), self._s()))
+        if self._numpy_io:
+            return (None if sx is None else sx[0].cpu().numpy()), su[0].cpu().numpy()
+        return sx, su
 
     def solver_status(self):
         """per-vehicle (status, iters) of the last solve; the reference discards acados' status (quad_opt.py:333)"""
