@@ -151,6 +151,27 @@ int qmpc_iters_total(qmpc_handle_t h, long long *total, void *stream);
  * to that set.  Returns QMPC_ERR_ARG before the handle's first solve and for fp32 handles. */
 int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double *sens_x, double *sens_u, void *stream);
 
+/* Reverse mode of the same solution map, now w.r.t. x0 AND the reference, for every vehicle at once: for cotangents
+ * x_bar [B][N+1][13] and u_bar [B][N][4] of the last solve's x, u (either may be NULL = zero), the gradients of
+ * <x_bar, x> + <u_bar, u> w.r.t. x0 -> x0_bar [B][13], yref -> yref_bar [B][N][17] and yref_e -> yref_e_bar [B][13]
+ * (any of the three may be NULL; outputs are overwritten, not accumulated).  The linearisation reads the reference only
+ * in the linear cost term, so on the active set of the last solve these are exact: with (xh, uh) the minimiser of the
+ * pinned LQR with linear costs -x_bar, -u_bar from xh_0 = 0,  yref_bar[k] = (Qd xh_k, Rd uh_k) (Qd = dt w_diag[0:13],
+ * Rd = dt w_diag[13:17]; its stage-0 state part and pinned input entries are exactly 0), yref_e_bar = we_diag xh_N and
+ * x0_bar = sum_k sens_x[k]^T x_bar[k] + sens_u[k]^T u_bar[k].  Cotangents on pinned inputs have no effect.  NaN for
+ * vehicles whose active set is unknown.  With reset_on_fail on, a vehicle whose PREVIOUS solve failed was linearised
+ * at a point built from the reference: its result is the derivative at that fixed linearisation.  One pinned
+ * factorisation and two vector sweeps; reads the stage tiles and active set: valid until the next solve.  Asynchronous.
+ * Returns QMPC_ERR_ARG, launching nothing, before the handle's first solve, for fp32 handles, with both cotangents NULL
+ * and with all three outputs NULL. */
+int qmpc_eval_adjoint(qmpc_handle_t h, const double *x_bar, const double *u_bar, double *x0_bar, double *yref_bar,
+                      double *yref_e_bar, void *stream);
+
+/* host counter that changes whenever the data qmpc_eval_sens_x0 / qmpc_eval_adjoint read may change: every solve
+ * (qmpc_solve, qmpc_step, qmpc_step_dt, qmpc_closed_loop_step), qmpc_set_active_set and qmpc_reset_warm_start.  The
+ * sensitivity calls leave it alone.  A deferred backward compares it to refuse stale tiles. */
+int qmpc_get_sens_epoch(qmpc_handle_t h, long long *epoch);
+
 /* ---- stateless helpers of the loop (any B) */
 /* quad_optimizer.discrete_dynamics (quad_opt.py:353-377): nominal RK4 step, optional body-frame velocity.
  * x [B][13], u [B][4] -> x_next [B][13] */

@@ -82,6 +82,7 @@ struct qmpc_solver {
     std::vector<cudaEvent_t> ev;      // triples: before linearize, before ipm, after ipm
     std::vector<cudaEvent_t> ev_mid;  // between the screening and the dense kernel (one per timed solve)
     bool solved = false;              // a solve has been queued: the stage tiles W hold data (qmpc_eval_sens_x0)
+    long long epoch = 0;              // qmpc_get_sens_epoch: bumped whenever the tiles or the active set may change
 };
 
 struct qrgp_model {
@@ -157,6 +158,8 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
     CU_TRY(cudaFuncSetAttribute(qmpc_ipm_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem64));
     CU_TRY(cudaFuncSetAttribute(qmpc_ipm_kernel<float, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
     CU_TRY(cudaFuncSetAttribute(qmpc_sens_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
+    CU_TRY(cudaFuncSetAttribute(qmpc_adjoint_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     h->variant = solver_variant(h->cfg, DN_MAX_N);
     if (h->variant == 2) {
@@ -277,6 +280,7 @@ int qmpc_get_iterate(qmpc_handle_t h, double* x, double* u, void* stream)
 template <typename real>
 static int solve_impl(qmpc_solver* h, void* stream)
 {
+    ++h->epoch;                     // qmpc_solve, qmpc_step(_dt) and qmpc_closed_loop_step all come through here
     const int B = h->cfg.batch, N = h->cfg.n_nodes;
     LinArgs<double, real> la;       // the linearisation always runs in fp64; fp32 handles store fp32 tiles (see LinArgs)
     fill_lin_args(h->cfg, la);
@@ -356,6 +360,22 @@ static int sens_impl(qmpc_solver* h, int n_stages, double* sens_x, double* sens_
     return QMPC_OK;
 }
 
+static int adjoint_impl(qmpc_solver* h, const double* x_bar, const double* u_bar, double* x0_bar, double* yref_bar,
+                        double* yref_e_bar, void* stream)
+{
+    typedef double real;
+    const int B = h->cfg.batch;
+    AdjArgs<real> aa;
+    fill_sens_base(h->cfg, aa.b);
+    aa.b.x0 = nullptr; aa.b.yref = nullptr; aa.b.yref_e = h->yref_e; aa.b.xit = h->xit; aa.b.uit = nullptr;
+    aa.b.W = static_cast<const real*>(h->W); aa.b.fac = static_cast<real*>(h->fac); aa.b.act = h->act;
+    aa.x_bar = x_bar; aa.u_bar = u_bar; aa.x0_bar = x0_bar; aa.yref_bar = yref_bar; aa.yref_e_bar = yref_e_bar;
+    const size_t smem = (size_t)IPM_WARPS * aa.b.smem_per_warp * sizeof(real);
+    qmpc_adjoint_kernel<real, IPM_WARPS><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(aa);
+    LAUNCH_CHECK();
+    return QMPC_OK;
+}
+
 extern "C" {
 
 int qmpc_solve(qmpc_handle_t h, void* stream)
@@ -373,6 +393,24 @@ int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double* sens_x, double* sen
     if (h->cfg.precision != 64) return fail(QMPC_ERR_ARG, "sensitivities need an fp64 handle (precision 64)");
     if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
     return sens_impl(h, n_stages, sens_x, sens_u, stream);
+}
+
+int qmpc_eval_adjoint(qmpc_handle_t h, const double* x_bar, const double* u_bar, double* x0_bar, double* yref_bar,
+                      double* yref_e_bar, void* stream)
+{
+    if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    if (h->cfg.precision != 64) return fail(QMPC_ERR_ARG, "sensitivities need an fp64 handle (precision 64)");
+    if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
+    if (!x_bar && !u_bar) return fail(QMPC_ERR_ARG, "x_bar and u_bar are both NULL: nothing to differentiate");
+    if (!x0_bar && !yref_bar && !yref_e_bar) return fail(QMPC_ERR_ARG, "x0_bar, yref_bar and yref_e_bar are all NULL");
+    return adjoint_impl(h, x_bar, u_bar, x0_bar, yref_bar, yref_e_bar, stream);
+}
+
+int qmpc_get_sens_epoch(qmpc_handle_t h, long long* epoch)
+{
+    if (!h || !epoch) return fail(QMPC_ERR_ARG, "null argument");
+    *epoch = h->epoch;
+    return QMPC_OK;
 }
 
 int qmpc_get_u0(qmpc_handle_t h, double* u0, void* stream)
@@ -429,11 +467,13 @@ int qmpc_get_active_set(qmpc_handle_t h, unsigned char* act, void* stream)
 int qmpc_set_active_set(qmpc_handle_t h, const unsigned char* act, void* stream)
 {
     if (!h || !act) return fail(QMPC_ERR_ARG, "null argument");
+    ++h->epoch;
     return copy_dd(h->act, act, (size_t)h->cfg.batch * h->cfg.n_nodes * NU, stream);
 }
 int qmpc_reset_warm_start(qmpc_handle_t h, void* stream)
 {
     if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    ++h->epoch;
     CU_TRY(cudaMemsetAsync(h->act, 255, (size_t)h->cfg.batch * h->cfg.n_nodes * NU, S(stream)));
     return QMPC_OK;
 }

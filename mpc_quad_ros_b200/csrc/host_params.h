@@ -152,14 +152,21 @@ inline void fill_screen_args(const qmpc_config& c, IpmArgs<real>& a)
     a.refine_off = 0;
 }
 
-// qmpc_eval_sens_x0: weights of the solve, per-warp shared memory of the screening layout; the caller sets the pointers
+// qmpc_eval_sens_x0 / qmpc_eval_adjoint: weights of the solve, per-warp shared memory of the screening layout; the caller
+// sets the pointers
+template <typename real>
+inline void fill_sens_base(const qmpc_config& c, IpmArgs<real>& b)
+{
+    fill_ipm_args(c, b);
+    b.smem_per_warp = ipm_smem_reals(c.n_nodes, false, sizeof(real) == 8);
+    b.ring_off = ipm_ring_off(c.n_nodes, false);
+    b.refine_off = 0;
+}
+
 template <typename real>
 inline void fill_sens_args(const qmpc_config& c, int n_stages, SensArgs<real>& a)
 {
-    fill_ipm_args(c, a.b);
-    a.b.smem_per_warp = ipm_smem_reals(c.n_nodes, false, sizeof(real) == 8);
-    a.b.ring_off = ipm_ring_off(c.n_nodes, false);
-    a.b.refine_off = 0;
+    fill_sens_base(c, a.b);
     a.n_stages = n_stages;
 }
 

@@ -11,6 +11,8 @@
 //       iterate (SURVEY.md App. A.3).
 //   qmpc_sens_kernel      : behind qmpc_eval_sens_x0, not part of a solve: derivatives of the last solve's x[k], u[k] with
 //       respect to x0 (acados eval_param_sens "ex"), one OCP per warp from the tiles and the active set the solve left.
+//   qmpc_adjoint_kernel   : behind qmpc_eval_adjoint, not part of a solve: reverse mode of the same map, the gradients w.r.t.
+//       x0, yref and yref_e of <x_bar, x> + <u_bar, u> for given cotangents, one OCP per warp.
 //
 // Per-stage tile written by K1 and streamed by K2 (HBM/L2, `real`):   W[13 rows][16 cols], row stride WR
 //   cols 0..3  = B = dPhi/du            cols 4..13 = dPhi/dx_s for s = 3..12 (q,v,r)
@@ -1112,6 +1114,116 @@ struct WarpCtx {
             for (int i = 0; i < NX; ++i) dx[i] = xn[i];
         }
     }
+
+    // Backward half of the adjoint (reverse mode) of the pinned LQR whose factors backward_full<true>() left in `fac`:
+    // the gradient sweep of backward_vec<true> with the cotangents as linear costs, q_k = -xb_k on the states, r_k = -ub_k
+    // on the inputs (pinned inputs take none), p_N = -xb_N, no offsets.  Unlike backward_vec it carries the state terms
+    // and updates p at stage 0 as well: on return pv[0..12] = p_0, the costate of x_0, and x0_bar = -p_0.  lgc goes to
+    // fac[66..69] for forward_cotangent.  xb [(N+1)][13], ub [N][4]; either may be null (zero cotangent).
+    __device__ void backward_cotangent(const double* xb, const double* ub)
+    {
+        if (lane < 16) pv[lane] = (xb && lane < NX) ? real(-xb[(size_t)N * NX + lane]) : real(0);
+        __syncwarp();
+        sweep_begin(N - 1, -1);
+        for (int k = N - 1; k >= 0; --k) {
+            real w[NX];
+            load_col(tile_at(N - 1 - k, k), w);
+            prefetch_stage(k - 1, true);
+            const real* f = facv + (size_t)k * FAC;
+            Chol4<double> L;
+            L.load(f + 56);
+            real lx[4] = {0, 0, 0, 0};
+            if (sidx >= 0) { ld2(f + sidx * 4, lx[0], lx[1]); ld2(f + sidx * 4 + 2, lx[2], lx[3]); }
+            real g = 0;
+#pragma unroll
+            for (int c = 0; c < 12; c += 2) {
+                real h0, h1;
+                ld2(pv + c, h0, h1);
+                g += w[c] * h0 + w[c + 1] * h1;
+            }
+            g += w[12] * pv[12];
+            if (j < 4 && ub) g -= real(ub[k * 4 + j]);
+            const real qs = (sidx >= 0 && xb) ? real(-xb[(size_t)k * NX + sidx]) : real(0);
+            real gu[4], lgc[4];
+#pragma unroll
+            for (int aa = 0; aa < 4; ++aa) gu[aa] = __shfl_sync(FULL, g, aa);
+#pragma unroll
+            for (int aa = 0; aa < 4; ++aa) if (fx[k * 4 + aa] != real(0)) gu[aa] = 0;
+            L.fsolve(gu, lgc);
+            const real pold = j < 3 ? pv[j] : real(0);
+            __syncwarp();
+            tile_done(N - 1 - k, k - RING);
+            if (h == 0) {
+                if (j >= 4 && j < 14) pv[j - 1] = g + qs - dot4(lx, lgc);
+                else if (j < 3) pv[j] = pold + qs - dot4(lx, lgc);
+                else if (j == 14) {
+#pragma unroll
+                    for (int aa = 0; aa < 4; ++aa) facv[(size_t)k * FAC + 66 + aa] = lgc[aa];
+                }
+            }
+            __syncwarp();
+        }
+    }
+
+    // Forward half of the adjoint: the minimiser of that LQR from x_0 = 0, du_k = -Lam^-T (Lx dx_k + lgc_k) (pinned
+    // entries 0), dx_{k+1} = A dx_k + B du_k, contracted with the cost weights as it goes: yb[k] = (Qd dx_k, Rd du_k),
+    // yeb = QNd dx_N.  Every lane carries the whole state (tile rows and factor records are broadcasts, as in
+    // forward_sens); lanes 0..16 store one entry of yb[k] each, lanes 0..12 one of yeb.  yb [N][17], yeb [13] or null.
+    __device__ void forward_cotangent(double* yb, double* yeb)
+    {
+        real dx[NX];
+#pragma unroll
+        for (int i = 0; i < NX; ++i) dx[i] = 0;
+        sweep_begin(0, 1);
+        for (int k = 0; k < N; ++k) {
+            const real* t = tile_at(k, k);
+            const real* f = facv + (size_t)k * FAC;
+            Chol4<double> L;
+            L.load(f + 56);
+            real v[4];
+            ld2(f + 66, v[0], v[1]); ld2(f + 68, v[2], v[3]);
+#pragma unroll
+            for (int s_ = 0; s_ < NX; ++s_) {
+                real l0, l1, l2, l3;
+                ld2(f + s_ * 4, l0, l1); ld2(f + s_ * 4 + 2, l2, l3);
+                v[0] = fma(l0, dx[s_], v[0]); v[1] = fma(l1, dx[s_], v[1]);
+                v[2] = fma(l2, dx[s_], v[2]); v[3] = fma(l3, dx[s_], v[3]);
+            }
+            real du[4];
+            L.bsolve_neg(v, du);
+#pragma unroll
+            for (int aa = 0; aa < 4; ++aa) if (fx[k * 4 + aa] != real(0)) du[aa] = 0;
+            real xn[NX];
+#pragma unroll
+            for (int i = 0; i < NX; ++i) {
+                const real* row = t + i * WR;
+                real acc = i < 3 ? dx[i] : real(0);             // position columns of A: unit vectors, not stored
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) acc = fma(tld(row + aa), du[aa], acc);
+#pragma unroll
+                for (int s_ = 3; s_ < NX; ++s_) acc = fma(tld(row + 1 + s_), dx[s_], acc);
+                xn[i] = acc;
+            }
+            __syncwarp();                       // every lane has read the tile
+            tile_done(k, k + RING);
+            if (yb) {
+                real mine = 0;                  // selects on the lane index, not a run-time index into the register arrays
+#pragma unroll
+                for (int i = 0; i < NX; ++i) if (lane == i) mine = a.Qd[i] * dx[i];
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) if (lane == NX + aa) mine = a.Rd[aa] * du[aa];
+                if (lane < NY) yb[k * NY + lane] = double(mine);
+            }
+#pragma unroll
+            for (int i = 0; i < NX; ++i) dx[i] = xn[i];
+        }
+        if (yeb) {
+            real mine = 0;
+#pragma unroll
+            for (int i = 0; i < NX; ++i) if (lane == i) mine = a.QNd[i] * dx[i];
+            if (lane < NX) yeb[lane] = double(mine);
+        }
+    }
 };
 
 #ifndef QMPC_IPM_MIN_WARPS
@@ -1480,6 +1592,98 @@ __global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_sens_
     c.template backward_full<true>();
     c.N = ns;              // the sweep streams stages 0..ns-1 only: no tile copy is in flight when the warp exits
     c.forward_sens(sx, su);
+}
+
+// ------------------------------------------------------------------------------------------ adjoint sensitivities
+
+// Set-up of qmpc_adjoint_kernel for one OCP, the same as qmpc_sens_kernel's (that kernel keeps its inline copy: moved into
+// this function it compiles to a different register allocation): the warp context of qmpc_ipm_kernel in its screening
+// layout, then the pinned factorisation of the active-set rounds (backward_full<true>) on the active set `act` of the
+// last solve.  The sweeps that follow read the per-warp work space, rdel, fx, fv, the tiles, `fac`, and xit / yref_e
+// for the (unused) costate offset.
+template <typename real>
+__device__ __forceinline__ void sens_factorise(WarpCtx<real>& c, unsigned char* smem_raw, int warp, int lane, int ocp,
+                                               const unsigned char* act)
+{
+    const IpmArgs<real>& a = c.a;
+    const int N = a.N, E = 4 * N;
+    real* sm = reinterpret_cast<real*>(smem_raw) + (size_t)warp * a.smem_per_warp;
+    c.lane = lane; c.h = lane >> 4; c.j = lane & 15; c.ocp = ocp; c.N = N; c.E = E;
+    c.hmask = 0xffffu << (lane & 16);
+    c.sidx = (c.j < 3) ? c.j : ((c.j >= 4 && c.j < 14) ? c.j - 1 : -1);
+    c.P = sm + SM_P; c.pv = sm + SM_PV; c.wv = sm + SM_WV; c.xp = sm + SM_XP; c.hv = sm + SM_HV;
+    c.Ls = sm + SM_LS; c.cs = sm + SM_CS;
+    real* v = sm + SM_VEC;
+    c.usol = c.ua = c.ucur = c.ubar = c.grad = v; c.rdel = v + 3 * E; c.cl = v + 4 * E; c.cu = v + 5 * E;
+    c.xtr = v + 6 * E;
+    c.rt = c.dR = c.ll = c.lu = c.tl = c.tu = v;
+    c.fx = c.cl; c.fv = c.cu;
+    c.hist_store = sm + a.ring_off;
+    c.ring = sm + a.ring_off + HIST_REALS<real>();
+    c.rbar = reinterpret_cast<unsigned long long*>(c.ring + WarpCtx<real>::RING * WT);
+    c.rphase = 0;
+    c.gave_up = false;
+    if (WarpCtx<real>::RING) {
+        if (lane == 0) for (int s_ = 0; s_ < WarpCtx<real>::RING; ++s_) mbar_init(c.rbar + s_, 1);
+        __syncwarp();
+    }
+    c.Wv = a.W + (size_t)ocp * N * WT;
+    c.facv = a.fac + (size_t)ocp * N * FAC;
+    c.x0 = nullptr; c.yref = nullptr; c.uit = nullptr;
+    c.yref_e = a.yref_e + (size_t)ocp * NX;
+    c.xit = a.xit + (size_t)ocp * (N + 1) * NX;
+    // homogeneous problem: pinned inputs at 0, no input gradient (the offsets only reach lg / p, never the factors)
+    for (int e = lane; e < E; e += 32) { c.fx[e] = real(act[e]); c.fv[e] = 0; c.rdel[e] = 0; }
+    __syncwarp();
+    c.template backward_full<true>();
+}
+
+template <typename real>
+struct AdjArgs {
+    IpmArgs<real> b;           // as SensArgs::b
+    const double* x_bar;       // [B][N+1][13] cotangent of the states, or null (zero)
+    const double* u_bar;       // [B][N][4] cotangent of the inputs, or null (zero)
+    double* x0_bar;            // [B][13] or null
+    double* yref_bar;          // [B][N][17] or null
+    double* yref_e_bar;        // [B][13] or null
+};
+
+// Reverse mode of the same solution map, now also w.r.t. the reference: K1 reads the reference only in the linear cost
+// term (tile column 15, q = dt W_x (x_lin - xref)) and the solve only in rdel (from uref), so on the active set
+// d<xb, x> + <ub, u> = <x0_bar, dx0> + <yref_bar, dyref> + <yref_e_bar, dyref_e> with, for the minimiser (dx, du) of the
+// pinned LQR with linear costs -xb, -ub from dx_0 = 0:  yref_bar[k] = (Qd dx_k, Rd du_k), yref_e_bar = QNd dx_N and
+// x0_bar = -p_0, the costate of x_0.  One warp per OCP: sens_factorise, backward_cotangent, forward_cotangent (skipped
+// when neither reference output is wanted).  A vehicle whose active set is unknown gets NaN everywhere.
+// The fp64 factorisation spills at 16 resident warps as in qmpc_sens_kernel: the same register budget.
+template <typename real, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_adjoint_kernel(AdjArgs<real> s)
+{
+    QMPC_DYN_SMEM(smem_raw);
+    const IpmArgs<real>& a = s.b;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int ocp = blockIdx.x * WARPS + warp;
+    if (ocp >= a.B) return;
+    const int N = a.N, E = 4 * N;
+    const unsigned char* act = a.act + (size_t)ocp * E;
+    const double* xb = s.x_bar ? s.x_bar + (size_t)ocp * (N + 1) * NX : nullptr;
+    const double* ub = s.u_bar ? s.u_bar + (size_t)ocp * E : nullptr;
+    double* x0b = s.x0_bar ? s.x0_bar + (size_t)ocp * NX : nullptr;
+    double* yb = s.yref_bar ? s.yref_bar + (size_t)ocp * N * NY : nullptr;
+    double* yeb = s.yref_e_bar ? s.yref_e_bar + (size_t)ocp * NX : nullptr;
+    int known = 1;
+    for (int e = lane; e < E; e += 32) if (act[e] > 2) known = 0;
+    if (!warp_min(known)) {
+        const double qnan = nan("");
+        if (x0b && lane < NX) x0b[lane] = qnan;
+        if (yeb && lane < NX) yeb[lane] = qnan;
+        if (yb) for (int i = lane; i < N * NY; i += 32) yb[i] = qnan;
+        return;
+    }
+    WarpCtx<real> c{a};
+    sens_factorise(c, smem_raw, warp, lane, ocp, act);
+    c.backward_cotangent(xb, ub);
+    if (x0b && lane < NX) x0b[lane] = -double(c.pv[lane]);
+    if (yb || yeb) c.forward_cotangent(yb, yeb);
 }
 
 }  // namespace qmpc

@@ -160,6 +160,47 @@ class quad_optimizer:
             return (None if sx is None else sx[0].cpu().numpy()), su[0].cpu().numpy()
         return sx, su
 
+    def eval_adjoint(self, x_bar=None, u_bar=None):
+        """Reverse mode of the last solve (qmpc_eval_adjoint): for cotangents x_bar [N+1,13] and u_bar [N,4] of its x_opt,
+        w_opt (None = zero; batched: a leading B), the gradients of <x_bar, x_opt> + <u_bar, w_opt> w.r.t. x0, yref and
+        yref_N at the active set that solve ended on.  returns (x0_bar [13], yref_bar [N,17], yref_N_bar [13]); batched:
+        CUDA tensors with a leading B.  NaN for vehicles whose active set is unknown.  Valid until the next solve;
+        fp64 handles only (QmpcError otherwise)."""
+        x0b, yb, yeb = self._adjoint(x_bar, u_bar)
+        if self._numpy_io:
+            return x0b[0].cpu().numpy(), yb[0].cpu().numpy(), yeb[0].cpu().numpy()
+        return x0b, yb, yeb
+
+    def _adjoint(self, x_bar, u_bar):
+        B, N = self.batch, self.n_nodes
+        xb = None if x_bar is None else self._dev(x_bar, (B, N + 1, 13))
+        ub = None if u_bar is None else self._dev(u_bar, (B, N, 4))
+        x0b = torch.empty((B, 13), dtype=torch.float64, device=self.device)
+        yb = torch.empty((B, N, 17), dtype=torch.float64, device=self.device)
+        yeb = torch.empty((B, 13), dtype=torch.float64, device=self.device)
+        _capi.check(_capi.lib().qmpc_eval_adjoint(self._h, _capi.ptr(xb), _capi.ptr(ub), _capi.ptr(x0b), _capi.ptr(yb),
+                                                  _capi.ptr(yeb), self._s()))
+        return x0b, yb, yeb
+
+    def sens_epoch(self):
+        """qmpc_get_sens_epoch: changes with every solve (also the fused steps) and every set / reset of the active set"""
+        e = C.c_longlong()
+        _capi.check(_capi.lib().qmpc_get_sens_epoch(self._h, C.byref(e)))
+        return e.value
+
+    def differentiable_step(self, x0, x_ref, u_ref=None, iterate=None):
+        """set_reference_trajectory(x_ref, u_ref), optionally set_iterate(*iterate), run_optimization(x0) as a function
+        torch.autograd can differentiate w.r.t. x0 [B,13], x_ref [B,N,13] and u_ref [B,N,4] (tensors; no leading B for
+        batch 1 is accepted too).  returns (x_opt [B,N+1,13], u_opt [B,N,4]).  The backward is eval_adjoint: exact on
+        the active set of this solve; the iterate is the linearisation point and counts as a constant.  The backward
+        must run before the handle solves again or has its active set changed (RuntimeError otherwise).  With
+        reset_on_fail on, a vehicle whose previous solve failed is linearised at a point built from the reference: its
+        gradient is the one at that fixed linearisation."""
+        if iterate is not None and any(torch.is_tensor(t) and t.requires_grad for t in iterate):
+            raise ValueError("differentiable_step: the iterate is the linearisation point and is not differentiated; "
+                             "pass it detached")
+        return _RTIStep.apply(self, x0, x_ref, u_ref, iterate)
+
     def solver_status(self):
         """per-vehicle (status, iters) of the last solve; the reference discards acados' status (quad_opt.py:333)"""
         st = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
@@ -245,3 +286,36 @@ class quad_optimizer:
         _capi.check(_capi.lib().qmpc_step_dt(self._h, g, _capi.ptr(x_now), _capi.ptr(x_ref), _capi.ptr(x_pred_prev),
                                              int(bool(first_step)), _capi.ptr(u0_out),
                                              C.c_double(0.0 if odometry_dt is None else float(odometry_dt)), self._s()))
+
+
+class _RTIStep(torch.autograd.Function):
+    """quad_optimizer.differentiable_step: forward = one RTI solve, backward = qmpc_eval_adjoint on that solve's tiles"""
+
+    @staticmethod
+    def forward(ctx, opt, x0, x_ref, u_ref, iterate):
+        B, N = opt.batch, opt.n_nodes
+        opt.set_reference_trajectory(x_ref.detach().to(opt.device, torch.float64).reshape(B, N, 13),
+                                     None if u_ref is None else u_ref.detach().to(opt.device, torch.float64).reshape(B, N, 4))
+        if iterate is not None:
+            opt.set_iterate(*iterate)
+        x, u, _, _ = opt.run_optimization(x0.detach().to(opt.device, torch.float64).reshape(B, 13))
+        ctx.opt, ctx.epoch = opt, opt.sens_epoch()
+        ctx.like = [None if t is None else (t.shape, t.device, t.dtype) for t in (x0, x_ref, u_ref)]
+        ctx.set_materialize_grads(False)
+        lead = x0.shape[:-1]
+        return x.reshape(*lead, N + 1, 13), u.reshape(*lead, N, 4)
+
+    @staticmethod
+    def backward(ctx, x_bar, u_bar):
+        opt = ctx.opt
+        if x_bar is None and u_bar is None:
+            return None, None, None, None, None
+        if opt.sens_epoch() != ctx.epoch:
+            raise RuntimeError("differentiable_step: the handle has solved again or had its active set changed since "
+                               "this step's forward; the stage tiles and active set its backward needs are gone")
+        x0b, yb, yeb = opt._adjoint(x_bar, u_bar)
+        N = opt.n_nodes
+        x_ref_bar = yb[..., :13].clone()
+        x_ref_bar[:, N - 1] += yeb                     # yref_e = x_ref[:, N-1] (set_reference_kernel)
+        like = lambda g, i: g.reshape(ctx.like[i][0]).to(ctx.like[i][1], ctx.like[i][2]) if ctx.needs_input_grad[i + 1] else None
+        return None, like(x0b, 0), like(x_ref_bar, 1), like(yb[..., 13:], 2), None

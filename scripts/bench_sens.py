@@ -1,9 +1,12 @@
-"""Cost of qmpc_eval_sens_x0 (derivatives of the RTI step w.r.t. x0) beside the solve it differentiates.
+"""Cost of qmpc_eval_sens_x0 (derivatives of the RTI step w.r.t. x0) and of qmpc_eval_adjoint (its reverse mode, w.r.t. x0
+and the reference) beside the solve they differentiate.
 
 Workload: bench.py's random_smooth closed loop, B = 4096, N = 20, M = 20, fp64; 40 fused closed-loop steps first (the
 last 20 with qmpc_timing_* on, for the solve time), then 200 timed calls of each case with CUDA events around every call:
   gain    n_stages = 1 without states (K0 = du0/dx0 and nothing else)
   full    n_stages = N with states
+  adjoint       qmpc_eval_adjoint with u_bar on stage 0 only (x_bar NULL), all three outputs
+  adjoint_full  qmpc_eval_adjoint with every cotangent (x_bar and u_bar), all three outputs
 Prints one JSON line and writes it to --out.  Needs a GPU.
 
     python scripts/bench_sens.py --out bench_outputs/sens.json
@@ -93,6 +96,33 @@ def main():
         finite = bool(torch.isfinite(sun[ok]).all()) and (sxp is None or bool(torch.isfinite(sx[ok]).all()))
         out[name] = {"n_stages": n, "states": sxp is not None, "median_ms": float(np.median(t)),
                      "p99_ms": float(np.percentile(t, 99)), "min_ms": float(t.min()),
+                     "vehicles_status_ok": int(ok.sum().item()), "finite_for_status_ok": finite}
+
+    g = torch.Generator(device=dev).manual_seed(5)
+    xb = torch.randn((B, N + 1, 13), dtype=torch.float64, device=dev, generator=g)
+    ub = torch.randn((B, N, 4), dtype=torch.float64, device=dev, generator=g)
+    ub0 = torch.zeros_like(ub)
+    ub0[:, 0] = ub[:, 0]
+    x0b = torch.empty((B, 13), dtype=torch.float64, device=dev)
+    yb = torch.empty((B, N, 17), dtype=torch.float64, device=dev)
+    yeb = torch.empty((B, 13), dtype=torch.float64, device=dev)
+    adj = {"adjoint": (None, ub0), "adjoint_full": (xb, ub)}
+    for name, (xbp, ubp) in adj.items():
+        call = lambda: _capi.check(lib.qmpc_eval_adjoint(opt._h, _capi.ptr(xbp), _capi.ptr(ubp), _capi.ptr(x0b),
+                                                         _capi.ptr(yb), _capi.ptr(yeb), s))
+        for _ in range(10):
+            call()
+        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.calls)]
+        for e0, e1 in ev:
+            e0.record()
+            call()
+            e1.record()
+        torch.cuda.synchronize()
+        t = np.array([e0.elapsed_time(e1) for e0, e1 in ev])
+        ok = opt.solver_status()[0] == 0
+        finite = all(bool(torch.isfinite(o[ok]).all()) for o in (x0b, yb, yeb))
+        out[name] = {"x_bar": xbp is not None, "u_bar": "stage 0" if name == "adjoint" else "all",
+                     "median_ms": float(np.median(t)), "p99_ms": float(np.percentile(t, 99)), "min_ms": float(t.min()),
                      "vehicles_status_ok": int(ok.sum().item()), "finite_for_status_ok": finite}
     line = json.dumps(out)
     print(line)
