@@ -33,8 +33,13 @@ extern "C" {
 #define QMPC_ERR_CUDA (-2)
 #define QMPC_ERR_ALLOC (-3)
 
+/* longest horizon an fp32 handle (qmpc_config.precision = 32) accepts: past it the fp32 Riccati recursion and its three
+ * fp64 refinement steps leave the controls up to 1e-3 (dt = 1/N) and 2.5e-2 (dt = 0.01, N = 256) off the exact
+ * minimiser while its active set still verifies; up to 64 nodes they stay within 1e-4 */
+#define QMPC_FP32_MAX_NODES 64
+
 /* per-vehicle solver status written by qmpc_solve */
-#define QMPC_STATUS_OK 0        /* exact active set verified, or IPM converged below ipm_mu_tol */
+#define QMPC_STATUS_OK 0        /* exact active set verified (refine_max_rounds < 0: IPM below ipm_mu_tol) */
 #define QMPC_STATUS_MAXITER 1   /* ipm_max_iter reached (reference: qp_solver_iter_max = 50)  */
 #define QMPC_STATUS_NAN 2       /* NaN/Inf met                                                */
 
@@ -47,7 +52,7 @@ typedef struct {
     int batch;           /* B vehicles handled by this handle                                        */
     int n_nodes;         /* N (acados dims.N, quad_opt.py:98)                                        */
     int n_basis;         /* M RGP basis points per axis; 0 = nominal model (gpe=None)                */
-    int precision;       /* 64: fp64 solver (default) ; 32: fp32 Riccati/IPM (RGP stays fp64)        */
+    int precision;       /* 64: fp64 solver (default) ; 32: fp32 Riccati/IPM (RGP stays fp64), n_nodes <= QMPC_FP32_MAX_NODES */
     int device;          /* CUDA device ordinal                                                       */
     int ipm_max_iter;    /* <=0 -> 50                                                                  */
     int refine_max_rounds; /* active-set refinement rounds after the IPM: 0 -> 20 (fp32: 10), <0 -> off     */

@@ -117,6 +117,8 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
     if (cfg->batch < 1 || cfg->n_nodes < 1 || cfg->n_nodes > 256) return fail(QMPC_ERR_ARG, "batch/n_nodes out of range");
     if (cfg->n_basis < 0 || cfg->n_basis > 128) return fail(QMPC_ERR_ARG, "n_basis must be in [0,128]");
     if (cfg->precision != 64 && cfg->precision != 32 && cfg->precision != 0) return fail(QMPC_ERR_ARG, "precision must be 64 or 32");
+    if (cfg->precision == 32 && cfg->n_nodes > QMPC_FP32_MAX_NODES)
+        return fail(QMPC_ERR_ARG, "fp32 handles (precision 32) take n_nodes <= QMPC_FP32_MAX_NODES (64)");
     if (cfg->n_basis > 0 && !cfg->gp_X) return fail(QMPC_ERR_ARG, "gp_X is NULL with n_basis > 0");
     if (!(cfg->t_horizon > 0) || !(cfg->ubu > cfg->lbu)) return fail(QMPC_ERR_ARG, "t_horizon / bounds invalid");
     if (cfg->solver_variant < 0 || cfg->solver_variant > 2) return fail(QMPC_ERR_ARG, "solver_variant must be 0, 1 or 2");

@@ -1355,8 +1355,13 @@ __global__ void __launch_bounds__(WARPS * 32, QMPC_IPM_MIN_WARPS / WARPS) qmpc_i
                     for (int e = lane; e < E; e += 32)
                         c.fx[e] = c.tl[e] < c.ll[e] ? real(1) : (c.tu[e] < c.lu[e] ? real(2) : real(0));
                     if (c.refine_rounds(lb, ub, a.max_refine, rounds, a.post_bail != 0, a.bail_round)) { status = QMPC_STATUS_OK_; exact = true; break; }
-                    // inconsistent active set: one more attempt from a 100x sharper IPM point, then the IPM alone to mu_tol
+                    // inconsistent active set: one more attempt from a 100x sharper IPM point.  fp64: then a last one from
+                    // the IPM point at mu_tol; if that does not settle either, the IPM point is returned flagged MAXITER,
+                    // never as status 0 (it is not the minimiser: its distance grows as the dt-scaled multipliers shrink,
+                    // 3e-4 at N = 256).  fp32: the IPM alone to mu_tol, then the fp64-checked rounds below.
                     if (++attempts < 2) target *= real(1e-2);
+                    else if (sizeof(real) == 8 && attempts == 2) target = a.mu_tol;
+                    else if (sizeof(real) == 8) break;
                     else { refine = false; target = a.mu_tol; }
                     if (!refine && mu < target) { status = QMPC_STATUS_OK_; break; }
                 } else { status = QMPC_STATUS_OK_; break; }
