@@ -113,6 +113,13 @@ int qmpc_set_alpha(qmpc_handle_t h, const double *alpha, void *stream);
  * 3*M, or 0 when one shared model serves every vehicle); NULL returns to the handle's own storage.  Host-side switch,
  * takes effect for solves queued afterwards (used by the shared-swarm mode to double-buffer the model). */
 int qmpc_bind_alpha(qmpc_handle_t h, const double *alpha, int stride);
+/* replace the cost weights given at qmpc_create: w_diag [17] host (stage, diag(W)) and/or we_diag [13] host (terminal,
+ * diag(W_e)); NULL keeps that part.  Host-side, like qmpc_bind_alpha: takes effect for every solve queued afterwards
+ * (qmpc_solve, qmpc_step, qmpc_step_dt, qmpc_closed_loop_step); the iterate and the warm-start active sets are kept.
+ * qmpc_eval_sens_x0 / qmpc_eval_adjoint(_weights) keep using the weights of the last solve, and qmpc_get_sens_epoch does
+ * not change.  fp32 handles accept it.  Returns QMPC_ERR_ARG, changing nothing, with both arrays NULL and for a
+ * non-finite or negative entry or an input weight w_diag[13..16] that is not > 0. */
+int qmpc_set_weights(qmpc_handle_t h, const double *w_diag, const double *we_diag);
 /* persistent SQP iterate (acados keeps it inside the capsule; zero after create, SURVEY A.3):
  * x [B][N+1][13], u [B][N][4] */
 int qmpc_set_iterate(qmpc_handle_t h, const double *x, const double *u, void *stream);
@@ -162,7 +169,7 @@ int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double *sens_x, double *sen
  * (any of the three may be NULL; outputs are overwritten, not accumulated).  The linearisation reads the reference only
  * in the linear cost term, so on the active set of the last solve these are exact: with (xh, uh) the minimiser of the
  * pinned LQR with linear costs -x_bar, -u_bar from xh_0 = 0,  yref_bar[k] = (Qd xh_k, Rd uh_k) (Qd = dt w_diag[0:13],
- * Rd = dt w_diag[13:17]; its stage-0 state part and pinned input entries are exactly 0), yref_e_bar = we_diag xh_N and
+ * Rd = dt w_diag[13:17], the weights of the last solve; its stage-0 state part and pinned input entries are exactly 0), yref_e_bar = we_diag xh_N and
  * x0_bar = sum_k sens_x[k]^T x_bar[k] + sens_u[k]^T u_bar[k].  Cotangents on pinned inputs have no effect.  NaN for
  * vehicles whose active set is unknown.  With reset_on_fail on, a vehicle whose PREVIOUS solve failed was linearised
  * at a point built from the reference: its result is the derivative at that fixed linearisation.  One pinned
@@ -171,6 +178,21 @@ int qmpc_eval_sens_x0(qmpc_handle_t h, int n_stages, double *sens_x, double *sen
  * and with all three outputs NULL. */
 int qmpc_eval_adjoint(qmpc_handle_t h, const double *x_bar, const double *u_bar, double *x0_bar, double *yref_bar,
                       double *yref_e_bar, void *stream);
+
+/* qmpc_eval_adjoint plus the gradients of <x_bar, x> + <u_bar, u> w.r.t. the cost weights of the last solve, in one
+ * launch: w_bar [B][17] (w.r.t. w_diag) and we_bar [B][13] (w.r.t. we_diag), per vehicle; the weights are shared by the
+ * handle, so the gradient of a batch loss is their sum over vehicles.  The weights enter only the QP's objective, so on
+ * the active set of the last solve, with (xh, uh) as above and (x, u) that solve's solution (qmpc_get_x / qmpc_get_u):
+ *   w_bar[i] = -dt sum_k xh_k,i (x_k,i - yref_k,i) (i < 13),  w_bar[13+a] = -dt sum_k uh_k,a (u_k,a - yref_k,13+a),
+ *   we_bar[i] = -xh_N,i (x_N,i - yref_e_i).
+ * Scaling every weight by one factor leaves the solution unchanged, so sum_i w_diag[i] w_bar[i] + we_diag[i] we_bar[i]
+ * = 0 for every vehicle.  The first three outputs are bit-identical to qmpc_eval_adjoint's.  Any of the five outputs may
+ * be NULL.  Reads the handle's x, u and reference as well: valid until the next solve, qmpc_set_iterate, qmpc_set_yref
+ * or qmpc_set_reference.  The reset_on_fail caveat does not apply to w_bar / we_bar: the reset iterate is built from
+ * the reference, not from the weights.  NaN in all five for vehicles whose active set is unknown.  Asynchronous.
+ * Returns QMPC_ERR_ARG, launching nothing, in the cases of qmpc_eval_adjoint and with all five outputs NULL. */
+int qmpc_eval_adjoint_weights(qmpc_handle_t h, const double *x_bar, const double *u_bar, double *x0_bar,
+                              double *yref_bar, double *yref_e_bar, double *w_bar, double *we_bar, void *stream);
 
 /* host counter that changes whenever the data qmpc_eval_sens_x0 / qmpc_eval_adjoint read may change: every solve
  * (qmpc_solve, qmpc_step, qmpc_step_dt, qmpc_closed_loop_step), qmpc_set_active_set and qmpc_reset_warm_start.  The

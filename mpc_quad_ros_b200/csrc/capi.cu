@@ -83,6 +83,7 @@ struct qmpc_solver {
     std::vector<cudaEvent_t> ev_mid;  // between the screening and the dense kernel (one per timed solve)
     bool solved = false;              // a solve has been queued: the stage tiles W hold data (qmpc_eval_sens_x0)
     long long epoch = 0;              // qmpc_get_sens_epoch: bumped whenever the tiles or the active set may change
+    double w_solved[NY] = {}, we_solved[NX] = {};   // the weights the last solve ran with (cfg holds those of the next solve)
 };
 
 struct qrgp_model {
@@ -162,6 +163,8 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
     CU_TRY(cudaFuncSetAttribute(qmpc_sens_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     CU_TRY(cudaFuncSetAttribute(qmpc_adjoint_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
+    CU_TRY(cudaFuncSetAttribute(qmpc_adjoint_kernel<double, IPM_WARPS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     h->variant = solver_variant(h->cfg, DN_MAX_N);
     if (h->variant == 2) {
@@ -257,6 +260,22 @@ int qmpc_bind_alpha(qmpc_handle_t h, const double* alpha, int stride)
     return QMPC_OK;
 }
 
+int qmpc_set_weights(qmpc_handle_t h, const double* w_diag, const double* we_diag)
+{
+    if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    if (!w_diag && !we_diag) return fail(QMPC_ERR_ARG, "w_diag and we_diag are both NULL");
+    for (int i = 0; w_diag && i < NY; ++i) {
+        if (!std::isfinite(w_diag[i]) || w_diag[i] < 0) return fail(QMPC_ERR_ARG, "w_diag entries must be finite and >= 0");
+        // the Riccati and the dense factorisations need R positive definite
+        if (i >= NX && !(w_diag[i] > 0)) return fail(QMPC_ERR_ARG, "the input weights w_diag[13..16] must be > 0");
+    }
+    for (int i = 0; we_diag && i < NX; ++i)
+        if (!std::isfinite(we_diag[i]) || we_diag[i] < 0) return fail(QMPC_ERR_ARG, "we_diag entries must be finite and >= 0");
+    if (w_diag) std::memcpy(h->cfg.w_diag, w_diag, sizeof(h->cfg.w_diag));
+    if (we_diag) std::memcpy(h->cfg.we_diag, we_diag, sizeof(h->cfg.we_diag));
+    return QMPC_OK;
+}
+
 int qmpc_set_iterate(qmpc_handle_t h, const double* x, const double* u, void* stream)
 {
     if (!h) return fail(QMPC_ERR_ARG, "null handle");
@@ -283,6 +302,8 @@ template <typename real>
 static int solve_impl(qmpc_solver* h, void* stream)
 {
     ++h->epoch;                     // qmpc_solve, qmpc_step(_dt) and qmpc_closed_loop_step all come through here
+    std::memcpy(h->w_solved, h->cfg.w_diag, sizeof(h->w_solved));
+    std::memcpy(h->we_solved, h->cfg.we_diag, sizeof(h->we_solved));
     const int B = h->cfg.batch, N = h->cfg.n_nodes;
     LinArgs<double, real> la;       // the linearisation always runs in fp64; fp32 handles store fp32 tiles (see LinArgs)
     fill_lin_args(h->cfg, la);
@@ -347,12 +368,22 @@ static int solve_impl(qmpc_solver* h, void* stream)
     return QMPC_OK;
 }
 
+// the handle's configuration with the weights of its last solve: the sensitivities differentiate that solve, whatever
+// qmpc_set_weights has set for the next one
+static qmpc_config solved_cfg(const qmpc_solver* h)
+{
+    qmpc_config c = h->cfg;
+    std::memcpy(c.w_diag, h->w_solved, sizeof(c.w_diag));
+    std::memcpy(c.we_diag, h->we_solved, sizeof(c.we_diag));
+    return c;
+}
+
 static int sens_impl(qmpc_solver* h, int n_stages, double* sens_x, double* sens_u, void* stream)
 {
     typedef double real;
     const int B = h->cfg.batch;
     SensArgs<real> sa;
-    fill_sens_args(h->cfg, n_stages, sa);
+    fill_sens_args(solved_cfg(h), n_stages, sa);
     sa.b.x0 = nullptr; sa.b.yref = nullptr; sa.b.yref_e = h->yref_e; sa.b.xit = h->xit; sa.b.uit = nullptr;
     sa.b.W = static_cast<const real*>(h->W); sa.b.fac = static_cast<real*>(h->fac); sa.b.act = h->act;
     sa.sens_x = sens_x; sa.sens_u = sens_u;
@@ -362,18 +393,23 @@ static int sens_impl(qmpc_solver* h, int n_stages, double* sens_x, double* sens_
     return QMPC_OK;
 }
 
+// weights: qmpc_eval_adjoint_weights (w_bar / we_bar, the kernel's WGT instantiation); otherwise qmpc_eval_adjoint
 static int adjoint_impl(qmpc_solver* h, const double* x_bar, const double* u_bar, double* x0_bar, double* yref_bar,
-                        double* yref_e_bar, void* stream)
+                        double* yref_e_bar, bool weights, double* w_bar, double* we_bar, void* stream)
 {
     typedef double real;
     const int B = h->cfg.batch;
     AdjArgs<real> aa;
-    fill_sens_base(h->cfg, aa.b);
+    fill_sens_base(solved_cfg(h), aa.b);
     aa.b.x0 = nullptr; aa.b.yref = nullptr; aa.b.yref_e = h->yref_e; aa.b.xit = h->xit; aa.b.uit = nullptr;
     aa.b.W = static_cast<const real*>(h->W); aa.b.fac = static_cast<real*>(h->fac); aa.b.act = h->act;
     aa.x_bar = x_bar; aa.u_bar = u_bar; aa.x0_bar = x0_bar; aa.yref_bar = yref_bar; aa.yref_e_bar = yref_e_bar;
+    aa.x = h->xit; aa.u = h->uit; aa.yref = h->yref; aa.yref_e = h->yref_e; aa.w_bar = w_bar; aa.we_bar = we_bar;
     const size_t smem = (size_t)IPM_WARPS * aa.b.smem_per_warp * sizeof(real);
-    qmpc_adjoint_kernel<real, IPM_WARPS><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(aa);
+    if (weights)
+        qmpc_adjoint_kernel<real, IPM_WARPS, true><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(aa);
+    else
+        qmpc_adjoint_kernel<real, IPM_WARPS><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(aa);
     LAUNCH_CHECK();
     return QMPC_OK;
 }
@@ -405,7 +441,19 @@ int qmpc_eval_adjoint(qmpc_handle_t h, const double* x_bar, const double* u_bar,
     if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
     if (!x_bar && !u_bar) return fail(QMPC_ERR_ARG, "x_bar and u_bar are both NULL: nothing to differentiate");
     if (!x0_bar && !yref_bar && !yref_e_bar) return fail(QMPC_ERR_ARG, "x0_bar, yref_bar and yref_e_bar are all NULL");
-    return adjoint_impl(h, x_bar, u_bar, x0_bar, yref_bar, yref_e_bar, stream);
+    return adjoint_impl(h, x_bar, u_bar, x0_bar, yref_bar, yref_e_bar, false, nullptr, nullptr, stream);
+}
+
+int qmpc_eval_adjoint_weights(qmpc_handle_t h, const double* x_bar, const double* u_bar, double* x0_bar,
+                              double* yref_bar, double* yref_e_bar, double* w_bar, double* we_bar, void* stream)
+{
+    if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    if (h->cfg.precision != 64) return fail(QMPC_ERR_ARG, "sensitivities need an fp64 handle (precision 64)");
+    if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
+    if (!x_bar && !u_bar) return fail(QMPC_ERR_ARG, "x_bar and u_bar are both NULL: nothing to differentiate");
+    if (!x0_bar && !yref_bar && !yref_e_bar && !w_bar && !we_bar)
+        return fail(QMPC_ERR_ARG, "x0_bar, yref_bar, yref_e_bar, w_bar and we_bar are all NULL");
+    return adjoint_impl(h, x_bar, u_bar, x0_bar, yref_bar, yref_e_bar, true, w_bar, we_bar, stream);
 }
 
 int qmpc_get_sens_epoch(qmpc_handle_t h, long long* epoch)

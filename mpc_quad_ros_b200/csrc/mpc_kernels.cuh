@@ -12,7 +12,8 @@
 //   qmpc_sens_kernel      : behind qmpc_eval_sens_x0, not part of a solve: derivatives of the last solve's x[k], u[k] with
 //       respect to x0 (acados eval_param_sens "ex"), one OCP per warp from the tiles and the active set the solve left.
 //   qmpc_adjoint_kernel   : behind qmpc_eval_adjoint, not part of a solve: reverse mode of the same map, the gradients w.r.t.
-//       x0, yref and yref_e of <x_bar, x> + <u_bar, u> for given cotangents, one OCP per warp.
+//       x0, yref and yref_e of <x_bar, x> + <u_bar, u> for given cotangents, one OCP per warp; its WGT instantiation
+//       (qmpc_eval_adjoint_weights) adds the gradients w.r.t. the cost weights w_diag / we_diag.
 //
 // Per-stage tile written by K1 and streamed by K2 (HBM/L2, `real`):   W[13 rows][16 cols], row stride WR
 //   cols 0..3  = B = dPhi/du            cols 4..13 = dPhi/dx_s for s = 3..12 (q,v,r)
@@ -1169,11 +1170,19 @@ struct WarpCtx {
     // entries 0), dx_{k+1} = A dx_k + B du_k, contracted with the cost weights as it goes: yb[k] = (Qd dx_k, Rd du_k),
     // yeb = QNd dx_N.  Every lane carries the whole state (tile rows and factor records are broadcasts, as in
     // forward_sens); lanes 0..16 store one entry of yb[k] each, lanes 0..12 one of yeb.  yb [N][17], yeb [13] or null.
-    __device__ void forward_cotangent(double* yb, double* yeb)
+    // WGT (qmpc_eval_adjoint_weights): also the gradients w.r.t. the cost weights, from the last solve's solution xs
+    // [(N+1)][13], us [N][4] and the reference yr [N][17], yre [13]: lane i < 17 accumulates (dx_k, du_k)_i (z_k - yref_k)_i
+    // over k and stores wb[i] = -dt acc, lanes 0..12 store web[i] = -dx_N,i (x_N - yref_e)_i.  wb [17], web [13] or null.
+    // Each lane owns its entries: no cross-lane reduction, so the result is bit-reproducible.
+    template <bool WGT = false>
+    __device__ void forward_cotangent(double* yb, double* yeb, const double* xs = nullptr, const double* us = nullptr,
+                                      const double* yr = nullptr, const double* yre = nullptr, double* wb = nullptr,
+                                      double* web = nullptr)
     {
         real dx[NX];
 #pragma unroll
         for (int i = 0; i < NX; ++i) dx[i] = 0;
+        real wacc = 0;
         sweep_begin(0, 1);
         for (int k = 0; k < N; ++k) {
             const real* t = tile_at(k, k);
@@ -1214,6 +1223,16 @@ struct WarpCtx {
                 for (int aa = 0; aa < 4; ++aa) if (lane == NX + aa) mine = a.Rd[aa] * du[aa];
                 if (lane < NY) yb[k * NY + lane] = double(mine);
             }
+            if constexpr (WGT) {
+                real mine = 0, res = 0;
+#pragma unroll
+                for (int i = 0; i < NX; ++i) if (lane == i) mine = dx[i];
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) if (lane == NX + aa) mine = du[aa];
+                if (lane < NX) res = real(xs[k * NX + lane] - yr[k * NY + lane]);
+                else if (lane < NY) res = real(us[k * 4 + lane - NX] - yr[k * NY + lane]);
+                wacc = fma(mine, res, wacc);
+            }
 #pragma unroll
             for (int i = 0; i < NX; ++i) dx[i] = xn[i];
         }
@@ -1222,6 +1241,15 @@ struct WarpCtx {
 #pragma unroll
             for (int i = 0; i < NX; ++i) if (lane == i) mine = a.QNd[i] * dx[i];
             if (lane < NX) yeb[lane] = double(mine);
+        }
+        if constexpr (WGT) {
+            if (wb && lane < NY) wb[lane] = -double(a.dt * wacc);
+            if (web) {
+                real mine = 0;
+#pragma unroll
+                for (int i = 0; i < NX; ++i) if (lane == i) mine = dx[i];
+                if (lane < NX) web[lane] = -double(mine * real(xs[(size_t)N * NX + lane] - yre[lane]));
+            }
         }
     }
 };
@@ -1651,6 +1679,13 @@ struct AdjArgs {
     double* x0_bar;            // [B][13] or null
     double* yref_bar;          // [B][N][17] or null
     double* yref_e_bar;        // [B][13] or null
+    // read by the WGT instantiation only (qmpc_eval_adjoint_weights)
+    const double* x;           // [B][N+1][13] the last solve's states
+    const double* u;           // [B][N][4] the last solve's inputs
+    const double* yref;        // [B][N][17] the reference that solve ran with
+    const double* yref_e;      // [B][13]
+    double* w_bar;             // [B][17] gradient w.r.t. w_diag, or null
+    double* we_bar;            // [B][13] gradient w.r.t. we_diag, or null
 };
 
 // Reverse mode of the same solution map, now also w.r.t. the reference: K1 reads the reference only in the linear cost
@@ -1658,9 +1693,12 @@ struct AdjArgs {
 // d<xb, x> + <ub, u> = <x0_bar, dx0> + <yref_bar, dyref> + <yref_e_bar, dyref_e> with, for the minimiser (dx, du) of the
 // pinned LQR with linear costs -xb, -ub from dx_0 = 0:  yref_bar[k] = (Qd dx_k, Rd du_k), yref_e_bar = QNd dx_N and
 // x0_bar = -p_0, the costate of x_0.  One warp per OCP: sens_factorise, backward_cotangent, forward_cotangent (skipped
-// when neither reference output is wanted).  A vehicle whose active set is unknown gets NaN everywhere.
+// when no output it writes is wanted).  A vehicle whose active set is unknown gets NaN everywhere.
+// WGT: also the gradients w.r.t. the cost weights.  The weights enter the QP only through its objective (Hessian dt W,
+// tile column 15, rdel), never the linearisation, so with z the solution and (dx, du) the minimiser above,
+// w_bar[i] = -dt sum_k (dx_k, du_k)_i (z_k - yref_k)_i and we_bar[i] = -dx_N,i (x_N - yref_e)_i (DESIGN.md §4).
 // The fp64 factorisation spills at 16 resident warps as in qmpc_sens_kernel: the same register budget.
-template <typename real, int WARPS>
+template <typename real, int WARPS, bool WGT = false>
 __global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_adjoint_kernel(AdjArgs<real> s)
 {
     QMPC_DYN_SMEM(smem_raw);
@@ -1675,6 +1713,8 @@ __global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_adjoi
     double* x0b = s.x0_bar ? s.x0_bar + (size_t)ocp * NX : nullptr;
     double* yb = s.yref_bar ? s.yref_bar + (size_t)ocp * N * NY : nullptr;
     double* yeb = s.yref_e_bar ? s.yref_e_bar + (size_t)ocp * NX : nullptr;
+    double* wb = (WGT && s.w_bar) ? s.w_bar + (size_t)ocp * NY : nullptr;
+    double* web = (WGT && s.we_bar) ? s.we_bar + (size_t)ocp * NX : nullptr;
     int known = 1;
     for (int e = lane; e < E; e += 32) if (act[e] > 2) known = 0;
     if (!warp_min(known)) {
@@ -1682,13 +1722,23 @@ __global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_adjoi
         if (x0b && lane < NX) x0b[lane] = qnan;
         if (yeb && lane < NX) yeb[lane] = qnan;
         if (yb) for (int i = lane; i < N * NY; i += 32) yb[i] = qnan;
+        if constexpr (WGT) {
+            if (wb && lane < NY) wb[lane] = qnan;
+            if (web && lane < NX) web[lane] = qnan;
+        }
         return;
     }
     WarpCtx<real> c{a};
     sens_factorise(c, smem_raw, warp, lane, ocp, act);
     c.backward_cotangent(xb, ub);
     if (x0b && lane < NX) x0b[lane] = -double(c.pv[lane]);
-    if (yb || yeb) c.forward_cotangent(yb, yeb);
+    if constexpr (WGT) {
+        if (yb || yeb || wb || web)
+            c.template forward_cotangent<true>(yb, yeb, s.x + (size_t)ocp * (N + 1) * NX, s.u + (size_t)ocp * E,
+                                               s.yref + (size_t)ocp * N * NY, s.yref_e + (size_t)ocp * NX, wb, web);
+    } else {
+        if (yb || yeb) c.forward_cotangent(yb, yeb);
+    }
 }
 
 }  // namespace qmpc

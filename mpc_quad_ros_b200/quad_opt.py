@@ -160,27 +160,50 @@ class quad_optimizer:
             return (None if sx is None else sx[0].cpu().numpy()), su[0].cpu().numpy()
         return sx, su
 
-    def eval_adjoint(self, x_bar=None, u_bar=None):
+    def eval_adjoint(self, x_bar=None, u_bar=None, weights=False):
         """Reverse mode of the last solve (qmpc_eval_adjoint): for cotangents x_bar [N+1,13] and u_bar [N,4] of its x_opt,
         w_opt (None = zero; batched: a leading B), the gradients of <x_bar, x_opt> + <u_bar, w_opt> w.r.t. x0, yref and
         yref_N at the active set that solve ended on.  returns (x0_bar [13], yref_bar [N,17], yref_N_bar [13]); batched:
-        CUDA tensors with a leading B.  NaN for vehicles whose active set is unknown.  Valid until the next solve;
-        fp64 handles only (QmpcError otherwise)."""
-        x0b, yb, yeb = self._adjoint(x_bar, u_bar)
+        CUDA tensors with a leading B.  weights=True (qmpc_eval_adjoint_weights) appends the gradients w.r.t. the cost
+        weights of that solve, w_bar [17] (diag W) and we_bar [13] (diag W_e), per vehicle.  NaN for vehicles whose
+        active set is unknown.  Valid until the next solve (with weights=True also until the iterate or the reference
+        is set); fp64 handles only (QmpcError otherwise)."""
+        out = self._adjoint(x_bar, u_bar, weights)
         if self._numpy_io:
-            return x0b[0].cpu().numpy(), yb[0].cpu().numpy(), yeb[0].cpu().numpy()
-        return x0b, yb, yeb
+            return tuple(t[0].cpu().numpy() for t in out)
+        return out
 
-    def _adjoint(self, x_bar, u_bar):
+    def _adjoint(self, x_bar, u_bar, weights=False):
         B, N = self.batch, self.n_nodes
         xb = None if x_bar is None else self._dev(x_bar, (B, N + 1, 13))
         ub = None if u_bar is None else self._dev(u_bar, (B, N, 4))
         x0b = torch.empty((B, 13), dtype=torch.float64, device=self.device)
         yb = torch.empty((B, N, 17), dtype=torch.float64, device=self.device)
         yeb = torch.empty((B, 13), dtype=torch.float64, device=self.device)
-        _capi.check(_capi.lib().qmpc_eval_adjoint(self._h, _capi.ptr(xb), _capi.ptr(ub), _capi.ptr(x0b), _capi.ptr(yb),
-                                                  _capi.ptr(yeb), self._s()))
-        return x0b, yb, yeb
+        if not weights:
+            _capi.check(_capi.lib().qmpc_eval_adjoint(self._h, _capi.ptr(xb), _capi.ptr(ub), _capi.ptr(x0b),
+                                                      _capi.ptr(yb), _capi.ptr(yeb), self._s()))
+            return x0b, yb, yeb
+        wb = torch.empty((B, 17), dtype=torch.float64, device=self.device)
+        web = torch.empty((B, 13), dtype=torch.float64, device=self.device)
+        _capi.check(_capi.lib().qmpc_eval_adjoint_weights(self._h, _capi.ptr(xb), _capi.ptr(ub), _capi.ptr(x0b),
+                                                          _capi.ptr(yb), _capi.ptr(yeb), _capi.ptr(wb), _capi.ptr(web),
+                                                          self._s()))
+        return x0b, yb, yeb, wb, web
+
+    def set_weights(self, w_diag=None, we_diag=None):
+        """qmpc_set_weights: replace the stage weights diag(W) (17 entries) and/or the terminal weights diag(W_e) (13)
+        for every later solve; None keeps that part.  numpy arrays or tensors.  The iterate and the warm-start active
+        sets are kept; eval_sens / eval_adjoint keep differentiating the last solve with the weights it ran with."""
+        host = lambda a, n: None if a is None else np.ascontiguousarray(
+            (a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)), dtype=np.float64).reshape(n)
+        w, we = host(w_diag, 17), host(we_diag, 13)
+        p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        _capi.check(_capi.lib().qmpc_set_weights(self._h, p(w), p(we)))
+        if w is not None:
+            self.W = np.diag(w)
+        if we is not None:
+            self.W_e = np.diag(we)
 
     def sens_epoch(self):
         """qmpc_get_sens_epoch: changes with every solve (also the fused steps) and every set / reset of the active set"""
@@ -188,18 +211,21 @@ class quad_optimizer:
         _capi.check(_capi.lib().qmpc_get_sens_epoch(self._h, C.byref(e)))
         return e.value
 
-    def differentiable_step(self, x0, x_ref, u_ref=None, iterate=None):
+    def differentiable_step(self, x0, x_ref, u_ref=None, iterate=None, w_diag=None, we_diag=None):
         """set_reference_trajectory(x_ref, u_ref), optionally set_iterate(*iterate), run_optimization(x0) as a function
         torch.autograd can differentiate w.r.t. x0 [B,13], x_ref [B,N,13] and u_ref [B,N,4] (tensors; no leading B for
         batch 1 is accepted too).  returns (x_opt [B,N+1,13], u_opt [B,N,4]).  The backward is eval_adjoint: exact on
         the active set of this solve; the iterate is the linearisation point and counts as a constant.  The backward
         must run before the handle solves again or has its active set changed (RuntimeError otherwise).  With
         reset_on_fail on, a vehicle whose previous solve failed is linearised at a point built from the reference: its
-        gradient is the one at that fixed linearisation."""
+        gradient is the one at that fixed linearisation.
+        w_diag [17] / we_diag [13] (tensors, shared by every vehicle): the cost weights of this solve, set with
+        set_weights before it (they stay on the handle); differentiable too, their gradient is the sum over vehicles
+        of eval_adjoint(weights=True)'s w_bar / we_bar.  None keeps the handle's weights, which count as constants."""
         if iterate is not None and any(torch.is_tensor(t) and t.requires_grad for t in iterate):
             raise ValueError("differentiable_step: the iterate is the linearisation point and is not differentiated; "
                              "pass it detached")
-        return _RTIStep.apply(self, x0, x_ref, u_ref, iterate)
+        return _RTIStep.apply(self, x0, x_ref, u_ref, iterate, w_diag, we_diag)
 
     def solver_status(self):
         """per-vehicle (status, iters) of the last solve; the reference discards acados' status (quad_opt.py:333)"""
@@ -289,18 +315,22 @@ class quad_optimizer:
 
 
 class _RTIStep(torch.autograd.Function):
-    """quad_optimizer.differentiable_step: forward = one RTI solve, backward = qmpc_eval_adjoint on that solve's tiles"""
+    """quad_optimizer.differentiable_step: forward = one RTI solve, backward = qmpc_eval_adjoint (qmpc_eval_adjoint_weights
+    when the weights need a gradient) on that solve's tiles"""
 
     @staticmethod
-    def forward(ctx, opt, x0, x_ref, u_ref, iterate):
+    def forward(ctx, opt, x0, x_ref, u_ref, iterate, w_diag, we_diag):
         B, N = opt.batch, opt.n_nodes
+        if w_diag is not None or we_diag is not None:
+            opt.set_weights(w_diag, we_diag)
         opt.set_reference_trajectory(x_ref.detach().to(opt.device, torch.float64).reshape(B, N, 13),
                                      None if u_ref is None else u_ref.detach().to(opt.device, torch.float64).reshape(B, N, 4))
         if iterate is not None:
             opt.set_iterate(*iterate)
         x, u, _, _ = opt.run_optimization(x0.detach().to(opt.device, torch.float64).reshape(B, 13))
         ctx.opt, ctx.epoch = opt, opt.sens_epoch()
-        ctx.like = [None if t is None else (t.shape, t.device, t.dtype) for t in (x0, x_ref, u_ref)]
+        ctx.like = [(t.shape, t.device, t.dtype) if torch.is_tensor(t) else None
+                    for t in (x0, x_ref, u_ref, iterate, w_diag, we_diag)]
         ctx.set_materialize_grads(False)
         lead = x0.shape[:-1]
         return x.reshape(*lead, N + 1, 13), u.reshape(*lead, N, 4)
@@ -309,13 +339,16 @@ class _RTIStep(torch.autograd.Function):
     def backward(ctx, x_bar, u_bar):
         opt = ctx.opt
         if x_bar is None and u_bar is None:
-            return None, None, None, None, None
+            return None, None, None, None, None, None, None
         if opt.sens_epoch() != ctx.epoch:
             raise RuntimeError("differentiable_step: the handle has solved again or had its active set changed since "
                                "this step's forward; the stage tiles and active set its backward needs are gone")
-        x0b, yb, yeb = opt._adjoint(x_bar, u_bar)
+        weights = ctx.needs_input_grad[5] or ctx.needs_input_grad[6]
+        out = opt._adjoint(x_bar, u_bar, weights)
+        x0b, yb, yeb = out[:3]
         N = opt.n_nodes
         x_ref_bar = yb[..., :13].clone()
         x_ref_bar[:, N - 1] += yeb                     # yref_e = x_ref[:, N-1] (set_reference_kernel)
         like = lambda g, i: g.reshape(ctx.like[i][0]).to(ctx.like[i][1], ctx.like[i][2]) if ctx.needs_input_grad[i + 1] else None
-        return None, like(x0b, 0), like(x_ref_bar, 1), like(yb[..., 13:], 2), None
+        wb, web = (out[3].sum(0), out[4].sum(0)) if weights else (None, None)    # the weights are shared by the vehicles
+        return None, like(x0b, 0), like(x_ref_bar, 1), like(yb[..., 13:], 2), None, like(wb, 4), like(web, 5)
