@@ -64,7 +64,8 @@ typedef struct {
     double quad[20];     /* mass, max_thrust, J[3], x_f[4], y_f[4], z_l_tau[4], g[3]                  */
     double w_diag[17];   /* LINEAR_LS stage weights diag(W) (quad_opt.py:122-129); scaled by dt inside */
     double we_diag[13];  /* terminal weights diag(W_e) (quad_opt.py:130)                               */
-    double lbu, ubu;     /* input box (quad_opt.py:142-143)                                            */
+    double lbu, ubu;     /* input box (quad_opt.py:142-143): finite, lbu < ubu (QMPC_ERR_ARG otherwise: NaN or +-inf
+                            bounds are refused, since the IPM starts from the box centre 0.5 (lbu + ubu))       */
     double gp_theta[9];  /* per axis (L, sigma_f, sigma_n) (RGP.py:106)                                */
     const double *gp_X;  /* host [3][M] basis points, may be NULL when n_basis == 0.  Any layout is accepted; an axis
                             whose points are equispaced (linspace, what GPEnsemble.fromrange builds: GPE.py:127-150) is

@@ -121,7 +121,9 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
     if (cfg->precision == 32 && cfg->n_nodes > QMPC_FP32_MAX_NODES)
         return fail(QMPC_ERR_ARG, "fp32 handles (precision 32) take n_nodes <= QMPC_FP32_MAX_NODES (64)");
     if (cfg->n_basis > 0 && !cfg->gp_X) return fail(QMPC_ERR_ARG, "gp_X is NULL with n_basis > 0");
-    if (!(cfg->t_horizon > 0) || !(cfg->ubu > cfg->lbu)) return fail(QMPC_ERR_ARG, "t_horizon / bounds invalid");
+    // finite bounds only: the IPM starts from the box centre 0.5 (lbu + ubu)
+    if (!(cfg->t_horizon > 0) || !(cfg->ubu > cfg->lbu) || !std::isfinite(cfg->lbu) || !std::isfinite(cfg->ubu))
+        return fail(QMPC_ERR_ARG, "t_horizon / bounds invalid");
     if (cfg->solver_variant < 0 || cfg->solver_variant > 2) return fail(QMPC_ERR_ARG, "solver_variant must be 0, 1 or 2");
     if (cfg->solver_variant == 2 && (cfg->precision == 32 || cfg->n_nodes > DN_MAX_N))
         return fail(QMPC_ERR_ARG, "solver_variant 2 (screening + dense) needs fp64 and n_nodes <= 21");

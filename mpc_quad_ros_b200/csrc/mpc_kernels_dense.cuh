@@ -1033,8 +1033,12 @@ __global__ void __launch_bounds__(DN_THREADS, QMPC_DENSE_MIN_CTAS) qmpc_dense_ke
                     else if (!ipm_started) {     // the warm rounds did not settle: IPM from the box centre
                         DN_FOR_E(e) c.usol[e] = real(0.5) * (lb + ub) - c.ubar[e];
                         next = T_GRAD;
-                    } else {      // one more attempt from a 100x sharper IPM point, then the IPM alone
-                        if (++attempts < 2) target *= real(1e-2); else { refine = false; target = a.mu_tol; }
+                    } else if (++attempts < 3) {
+                        // one more attempt from a 100x sharper IPM point, then a last one from the IPM point at mu_tol (as
+                        // qmpc_ipm_kernel).  If that does not settle either, the IPM point is returned with status MAXITER
+                        // and flags 255, never as status 0: it is not the minimiser (1e-9..2e-8 off at N = 20 with
+                        // refine_max_rounds = 1, while its rounded active set already matched the exact one)
+                        target = attempts < 2 ? target * real(1e-2) : a.mu_tol;
                         next = T_PRED;
                     }
                 } else if (trip == T_PRED) {
