@@ -195,6 +195,24 @@ int qmpc_eval_adjoint(qmpc_handle_t h, const double *x_bar, const double *u_bar,
 int qmpc_eval_adjoint_weights(qmpc_handle_t h, const double *x_bar, const double *u_bar, double *x0_bar,
                               double *yref_bar, double *yref_e_bar, double *w_bar, double *we_bar, void *stream);
 
+/* Forward mode of the solution map of qmpc_eval_adjoint_weights: n_dir tangent directions per vehicle in one launch,
+ * all on one pinned factorisation.  Tangents dx0 [B][n_dir][13], dyref [B][n_dir][N][17], dyref_e [B][n_dir][13],
+ * dw [B][n_dir][17] (of w_diag) and dwe [B][n_dir][13] (of we_diag), device memory, any may be NULL (zero); outputs
+ * dx [B][n_dir][N+1][13] (may be NULL) and du [B][n_dir][N][4], overwritten.  On the active set of the last solve the
+ * step is linear in these tangents, and (dx, du) is exactly the minimiser of the pinned LQR of qmpc_eval_adjoint with
+ * dx_0 = dx0 and the linear costs  c_k = -dt w_diag (.) dyref_k + dt dw (.) (z_k - yref_k),
+ * c_N = -we_diag (.) dyref_e + dwe (.) (x_N - yref_e)  (z = (x, u) that solve's solution, the weights of that solve).
+ * So <x_bar, dx> + <u_bar, du> = <x0_bar, dx0> + <yref_bar, dyref> + <yref_e_bar, dyref_e> + <w_bar, dw> + <we_bar, dwe>
+ * with qmpc_eval_adjoint_weights' outputs, dx0 = e_i alone gives column i of qmpc_eval_sens_x0, and dw = w_diag,
+ * dwe = we_diag alone give 0.  du is exactly 0 on pinned inputs.  NaN in every output of every direction for vehicles
+ * whose active set is unknown.  The reset_on_fail caveat of qmpc_eval_adjoint applies to the x0 and reference
+ * directions, not to the weight directions.  Reads the stage tiles, the active set, x, u and the reference: valid until
+ * the next solve, qmpc_set_iterate, qmpc_set_yref or qmpc_set_reference.  Does not change qmpc_get_sens_epoch.
+ * Asynchronous.  Returns QMPC_ERR_ARG, launching nothing, before the handle's first solve, for fp32 handles, for
+ * n_dir < 1, with all five tangents NULL and with du NULL. */
+int qmpc_eval_jvp(qmpc_handle_t h, int n_dir, const double *dx0, const double *dyref, const double *dyref_e,
+                  const double *dw, const double *dwe, double *dx, double *du, void *stream);
+
 /* host counter that changes whenever the data qmpc_eval_sens_x0 / qmpc_eval_adjoint read may change: every solve
  * (qmpc_solve, qmpc_step, qmpc_step_dt, qmpc_closed_loop_step), qmpc_set_active_set and qmpc_reset_warm_start.  The
  * sensitivity calls leave it alone.  A deferred backward compares it to refuse stale tiles. */

@@ -43,6 +43,7 @@ def lib():
         L.qmpc_launch_count.restype = C.c_longlong
         L.qrgp_Kx_inv_device.restype = C.c_void_p
         L.qrgp_mu_device.restype = C.c_void_p
+        L.qmpc_eval_jvp.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
         _LIB = L
     return _LIB
 

@@ -168,6 +168,8 @@ int qmpc_create(const qmpc_config* cfg, qmpc_handle_t* out)
                                 IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     CU_TRY(cudaFuncSetAttribute(qmpc_adjoint_kernel<double, IPM_WARPS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
+    CU_TRY(cudaFuncSetAttribute(qmpc_jvp_kernel<double, IPM_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                IPM_WARPS * ipm_smem_reals((int)N, false, true) * 8));
     h->variant = solver_variant(h->cfg, DN_MAX_N);
     if (h->variant == 2) {
         const int smemd = dense_layout((int)N).total * 8;
@@ -416,6 +418,23 @@ static int adjoint_impl(qmpc_solver* h, const double* x_bar, const double* u_bar
     return QMPC_OK;
 }
 
+static int jvp_impl(qmpc_solver* h, int n_dir, const double* dx0, const double* dyref, const double* dyref_e,
+                    const double* dw, const double* dwe, double* dx, double* du, void* stream)
+{
+    typedef double real;
+    const int B = h->cfg.batch;
+    JvpArgs<real> ja;
+    fill_sens_base(solved_cfg(h), ja.b);
+    ja.b.x0 = nullptr; ja.b.yref = nullptr; ja.b.yref_e = h->yref_e; ja.b.xit = h->xit; ja.b.uit = nullptr;
+    ja.b.W = static_cast<const real*>(h->W); ja.b.fac = static_cast<real*>(h->fac); ja.b.act = h->act;
+    ja.K = n_dir; ja.dx0 = dx0; ja.dyref = dyref; ja.dyref_e = dyref_e; ja.dw = dw; ja.dwe = dwe; ja.dx = dx; ja.du = du;
+    ja.x = h->xit; ja.u = h->uit; ja.yref = h->yref; ja.yref_e = h->yref_e;
+    const size_t smem = (size_t)IPM_WARPS * ja.b.smem_per_warp * sizeof(real);
+    qmpc_jvp_kernel<real, IPM_WARPS><<<cdiv(B, IPM_WARPS), IPM_WARPS * 32, smem, S(stream)>>>(ja);
+    LAUNCH_CHECK();
+    return QMPC_OK;
+}
+
 extern "C" {
 
 int qmpc_solve(qmpc_handle_t h, void* stream)
@@ -456,6 +475,19 @@ int qmpc_eval_adjoint_weights(qmpc_handle_t h, const double* x_bar, const double
     if (!x0_bar && !yref_bar && !yref_e_bar && !w_bar && !we_bar)
         return fail(QMPC_ERR_ARG, "x0_bar, yref_bar, yref_e_bar, w_bar and we_bar are all NULL");
     return adjoint_impl(h, x_bar, u_bar, x0_bar, yref_bar, yref_e_bar, true, w_bar, we_bar, stream);
+}
+
+int qmpc_eval_jvp(qmpc_handle_t h, int n_dir, const double* dx0, const double* dyref, const double* dyref_e,
+                  const double* dw, const double* dwe, double* dx, double* du, void* stream)
+{
+    if (!h) return fail(QMPC_ERR_ARG, "null handle");
+    if (h->cfg.precision != 64) return fail(QMPC_ERR_ARG, "sensitivities need an fp64 handle (precision 64)");
+    if (!h->solved) return fail(QMPC_ERR_ARG, "no solve on this handle yet: the sensitivities need its stage tiles");
+    if (n_dir < 1) return fail(QMPC_ERR_ARG, "n_dir must be >= 1");
+    if (!dx0 && !dyref && !dyref_e && !dw && !dwe)
+        return fail(QMPC_ERR_ARG, "dx0, dyref, dyref_e, dw and dwe are all NULL: nothing to differentiate");
+    if (!du) return fail(QMPC_ERR_ARG, "du is NULL");
+    return jvp_impl(h, n_dir, dx0, dyref, dyref_e, dw, dwe, dx, du, stream);
 }
 
 int qmpc_get_sens_epoch(qmpc_handle_t h, long long* epoch)

@@ -14,6 +14,8 @@
 //   qmpc_adjoint_kernel   : behind qmpc_eval_adjoint, not part of a solve: reverse mode of the same map, the gradients w.r.t.
 //       x0, yref and yref_e of <x_bar, x> + <u_bar, u> for given cotangents, one OCP per warp; its WGT instantiation
 //       (qmpc_eval_adjoint_weights) adds the gradients w.r.t. the cost weights w_diag / we_diag.
+//   qmpc_jvp_kernel       : behind qmpc_eval_jvp, not part of a solve: forward mode of the same map w.r.t. x0, yref,
+//       yref_e and the cost weights, K tangent directions per vehicle on one pinned factorisation, one OCP per warp.
 //
 // Per-stage tile written by K1 and streamed by K2 (HBM/L2, `real`):   W[13 rows][16 cols], row stride WR
 //   cols 0..3  = B = dPhi/du            cols 4..13 = dPhi/dx_s for s = 3..12 (q,v,r)
@@ -449,6 +451,13 @@ constexpr int SM_VEC = 360;    // 13 vectors of 4N, then the state trajectory (N
 constexpr int SM_NVEC = 13;
 
 template <typename real> __host__ __device__ constexpr int HIST_REALS() { return 64 / (int)sizeof(real); }   // 64 bytes
+
+// One tangent direction of qmpc_eval_jvp and what its linear costs are formed from (WarpCtx::backward_cotangent<true>):
+// the tangents of the reference and the cost weights (any may be null = zero) and the last solve's solution and reference.
+struct TanDir {
+    const double *dyref, *dyref_e, *dw, *dwe;   // [N][17], [13], [17], [13]
+    const double *xs, *us, *yr, *yre;           // [(N+1)][13], [N][4], [N][17], [13]
+};
 
 template <typename real>
 struct WarpCtx {
@@ -1121,9 +1130,27 @@ struct WarpCtx {
     // on the inputs (pinned inputs take none), p_N = -xb_N, no offsets.  Unlike backward_vec it carries the state terms
     // and updates p at stage 0 as well: on return pv[0..12] = p_0, the costate of x_0, and x0_bar = -p_0.  lgc goes to
     // fac[66..69] for forward_cotangent.  xb [(N+1)][13], ub [N][4]; either may be null (zero cotangent).
-    __device__ void backward_cotangent(const double* xb, const double* ub)
+    // TAN (qmpc_eval_jvp): the linear costs are those of the forward mode for the direction t instead (xb, ub unused),
+    // formed per stage:  c_k = -(Qd, Rd) dyref_k + dt dw (z_k - yref_k),  c_N = -QNd dyref_e + dwe (x_N - yref_e)
+    // (DESIGN.md §4), i.e. the cotangents xb = -c_x, ub = -c_u.
+    template <bool TAN = false>
+    __device__ void backward_cotangent(const double* xb, const double* ub, const TanDir* t = nullptr)
     {
-        if (lane < 16) pv[lane] = (xb && lane < NX) ? real(-xb[(size_t)N * NX + lane]) : real(0);
+        real qd = 0, dq = 0, rd = 0, dr = 0;        // TAN: this lane's Hessian and dt dw entries of state sidx / input j
+        if constexpr (TAN) {
+            if (lane < 16) {
+                real pn = 0;
+                if (lane < NX) {
+                    if (t->dyref_e) pn = -a.QNd[lane] * real(t->dyref_e[lane]);
+                    if (t->dwe) pn = fma(real(t->dwe[lane]), real(t->xs[(size_t)N * NX + lane] - t->yre[lane]), pn);
+                }
+                pv[lane] = pn;
+            }
+            if (sidx >= 0) { qd = a.Qd[sidx]; if (t->dw) dq = a.dt * real(t->dw[sidx]); }
+            if (j < 4) { rd = a.Rd[j]; if (t->dw) dr = a.dt * real(t->dw[NX + j]); }
+        } else {
+            if (lane < 16) pv[lane] = (xb && lane < NX) ? real(-xb[(size_t)N * NX + lane]) : real(0);
+        }
         __syncwarp();
         sweep_begin(N - 1, -1);
         for (int k = N - 1; k >= 0; --k) {
@@ -1143,8 +1170,24 @@ struct WarpCtx {
                 g += w[c] * h0 + w[c + 1] * h1;
             }
             g += w[12] * pv[12];
-            if (j < 4 && ub) g -= real(ub[k * 4 + j]);
-            const real qs = (sidx >= 0 && xb) ? real(-xb[(size_t)k * NX + sidx]) : real(0);
+            real qs;
+            if constexpr (TAN) {
+                qs = 0;
+                const double* yk = t->yr + (size_t)k * NY;
+                if (j < 4) {
+                    real cu = 0;
+                    if (t->dyref) cu = -rd * real(t->dyref[(size_t)k * NY + NX + j]);
+                    if (t->dw) cu = fma(dr, real(t->us[k * 4 + j] - yk[NX + j]), cu);
+                    g += cu;
+                }
+                if (sidx >= 0) {
+                    if (t->dyref) qs = -qd * real(t->dyref[(size_t)k * NY + sidx]);
+                    if (t->dw) qs = fma(dq, real(t->xs[(size_t)k * NX + sidx] - yk[sidx]), qs);
+                }
+            } else {
+                if (j < 4 && ub) g -= real(ub[k * 4 + j]);
+                qs = (sidx >= 0 && xb) ? real(-xb[(size_t)k * NX + sidx]) : real(0);
+            }
             real gu[4], lgc[4];
 #pragma unroll
             for (int aa = 0; aa < 4; ++aa) gu[aa] = __shfl_sync(FULL, g, aa);
@@ -1174,14 +1217,29 @@ struct WarpCtx {
     // [(N+1)][13], us [N][4] and the reference yr [N][17], yre [13]: lane i < 17 accumulates (dx_k, du_k)_i (z_k - yref_k)_i
     // over k and stores wb[i] = -dt acc, lanes 0..12 store web[i] = -dx_N,i (x_N - yref_e)_i.  wb [17], web [13] or null.
     // Each lane owns its entries: no cross-lane reduction, so the result is bit-reproducible.
-    template <bool WGT = false>
+    // TAN (qmpc_eval_jvp): the roll-out starts from dx_0 = dx0 [13] (null = 0) and stores the tangent itself, dx_k to
+    // dxo [(N+1)][13] (or null) and du_k to duo [N][4]; yb, yeb must be null.
+    template <bool WGT = false, bool TAN = false>
     __device__ void forward_cotangent(double* yb, double* yeb, const double* xs = nullptr, const double* us = nullptr,
                                       const double* yr = nullptr, const double* yre = nullptr, double* wb = nullptr,
-                                      double* web = nullptr)
+                                      double* web = nullptr, const double* dx0 = nullptr, double* dxo = nullptr,
+                                      double* duo = nullptr)
     {
         real dx[NX];
 #pragma unroll
         for (int i = 0; i < NX; ++i) dx[i] = 0;
+        if constexpr (TAN) {
+            if (dx0) {
+#pragma unroll
+                for (int i = 0; i < NX; ++i) dx[i] = real(dx0[i]);
+            }
+            if (dxo) {
+                real mine = 0;
+#pragma unroll
+                for (int i = 0; i < NX; ++i) if (lane == i) mine = dx[i];
+                if (lane < NX) dxo[lane] = double(mine);
+            }
+        }
         real wacc = 0;
         sweep_begin(0, 1);
         for (int k = 0; k < N; ++k) {
@@ -1232,6 +1290,17 @@ struct WarpCtx {
                 if (lane < NX) res = real(xs[k * NX + lane] - yr[k * NY + lane]);
                 else if (lane < NY) res = real(us[k * 4 + lane - NX] - yr[k * NY + lane]);
                 wacc = fma(mine, res, wacc);
+            }
+            if constexpr (TAN) {
+                real mu = 0, mx = 0;
+#pragma unroll
+                for (int aa = 0; aa < 4; ++aa) if (lane == aa) mu = du[aa];
+                if (lane < NU) duo[k * NU + lane] = double(mu);
+                if (dxo) {
+#pragma unroll
+                    for (int i = 0; i < NX; ++i) if (lane == i) mx = xn[i];
+                    if (lane < NX) dxo[(size_t)(k + 1) * NX + lane] = double(mx);
+                }
             }
 #pragma unroll
             for (int i = 0; i < NX; ++i) dx[i] = xn[i];
@@ -1738,6 +1807,69 @@ __global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_adjoi
                                                s.yref + (size_t)ocp * N * NY, s.yref_e + (size_t)ocp * NX, wb, web);
     } else {
         if (yb || yeb) c.forward_cotangent(yb, yeb);
+    }
+}
+
+// ------------------------------------------------------------------------------------------ forward-mode sensitivities
+
+template <typename real>
+struct JvpArgs {
+    IpmArgs<real> b;           // as SensArgs::b
+    int K;                     // tangent directions per vehicle, >= 1
+    const double* dx0;         // [B][K][13] tangent of x0, or null (zero)
+    const double* dyref;       // [B][K][N][17] tangent of the reference, or null
+    const double* dyref_e;     // [B][K][13] or null
+    const double* dw;          // [B][K][17] tangent of w_diag, or null
+    const double* dwe;         // [B][K][13] tangent of we_diag, or null
+    double* dx;                // [B][K][N+1][13] or null
+    double* du;                // [B][K][N][4]
+    const double* x;           // [B][N+1][13] the last solve's states
+    const double* u;           // [B][N][4] the last solve's inputs
+    const double* yref;        // [B][N][17] the reference that solve ran with
+    const double* yref_e;      // [B][13]
+};
+
+// Forward mode of the solution map of qmpc_adjoint_kernel<.., true>: on the active set the solve ended on, the tangent
+// (dx, du) for (dx0, dyref, dyref_e, dw, dwe) is the minimiser of the pinned LQR of the adjoint with the linear costs
+// c_k = -(Qd, Rd) dyref_k + dt dw (z_k - yref_k), c_N = -QNd dyref_e + dwe (x_N - yref_e), from dx_0 = dx0 (DESIGN.md §4).
+// One warp per OCP: sens_factorise once, then per direction backward_cotangent<true> (costs formed per stage, nothing
+// stored) and forward_cotangent<false, true>; the K directions share the factorisation.  A vehicle whose active set is
+// unknown gets NaN in every output of every direction.  The same register budget as qmpc_adjoint_kernel.
+template <typename real, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, SENS_MIN_WARPS / WARPS) qmpc_jvp_kernel(JvpArgs<real> s)
+{
+    QMPC_DYN_SMEM(smem_raw);
+    const IpmArgs<real>& a = s.b;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int ocp = blockIdx.x * WARPS + warp;
+    if (ocp >= a.B) return;
+    const int N = a.N, E = 4 * N, K = s.K;
+    const unsigned char* act = a.act + (size_t)ocp * E;
+    double* dxo = s.dx ? s.dx + (size_t)ocp * K * (N + 1) * NX : nullptr;
+    double* duo = s.du + (size_t)ocp * K * E;
+    int known = 1;
+    for (int e = lane; e < E; e += 32) if (act[e] > 2) known = 0;
+    if (!warp_min(known)) {
+        const double qnan = nan("");
+        if (dxo) for (int i = lane; i < K * (N + 1) * NX; i += 32) dxo[i] = qnan;
+        for (int i = lane; i < K * E; i += 32) duo[i] = qnan;
+        return;
+    }
+    WarpCtx<real> c{a};
+    sens_factorise(c, smem_raw, warp, lane, ocp, act);
+    TanDir t;
+    t.xs = s.x + (size_t)ocp * (N + 1) * NX; t.us = s.u + (size_t)ocp * E;
+    t.yr = s.yref + (size_t)ocp * N * NY; t.yre = s.yref_e + (size_t)ocp * NX;
+    for (int d = 0; d < K; ++d) {
+        const size_t v = (size_t)ocp * K + d;          // (vehicle, direction)
+        t.dyref = s.dyref ? s.dyref + v * N * NY : nullptr;
+        t.dyref_e = s.dyref_e ? s.dyref_e + v * NX : nullptr;
+        t.dw = s.dw ? s.dw + v * NY : nullptr;
+        t.dwe = s.dwe ? s.dwe + v * NX : nullptr;
+        c.template backward_cotangent<true>(nullptr, nullptr, &t);
+        c.template forward_cotangent<false, true>(nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                                  s.dx0 ? s.dx0 + v * NX : nullptr,
+                                                  dxo ? dxo + (size_t)d * (N + 1) * NX : nullptr, duo + (size_t)d * E);
     }
 }
 

@@ -9,6 +9,7 @@ import time
 
 import numpy as np
 import torch
+import torch.autograd.forward_ad as fwAD
 
 from . import _capi
 from ._capi import QmpcConfig
@@ -191,6 +192,49 @@ class quad_optimizer:
                                                           self._s()))
         return x0b, yb, yeb, wb, web
 
+    def eval_jvp(self, dx0=None, dyref=None, dyref_e=None, dw=None, dwe=None):
+        """Forward mode of the last solve (qmpc_eval_jvp): the tangent (dx_opt, dw_opt) of its x_opt, w_opt for tangents of
+        x0 [B,K,13], yref [B,K,N,17], yref_N [B,K,13] and the cost weights of that solve, dw [B,K,17] (diag W) and
+        dwe [B,K,13] (diag W_e), at the active set that solve ended on; None = zero, at least one given.  The direction
+        axis K is optional (without it K = 1 and the outputs have none either); dw / dwe may also be [17] / [13], one
+        direction shared by every vehicle.  With numpy I/O (one vehicle, as the last run_optimization) the leading B is
+        absent.  The K directions share one pinned factorisation.  returns (dx [B,K,N+1,13], du [B,K,N,4]); batched:
+        CUDA tensors.  NaN for vehicles whose active set is unknown.  Valid until the next solve or until the iterate or
+        the reference is set; fp64 handles only (QmpcError otherwise)."""
+        out = self._jvp(dx0, dyref, dyref_e, dw, dwe, lead=0 if self._numpy_io else 1)
+        if self._numpy_io:
+            return tuple(t[0].cpu().numpy() for t in out)
+        return out
+
+    def _jvp(self, dx0, dyref, dyref_e, dw, dwe, lead=1):
+        """qmpc_eval_jvp; lead: the number of vehicle axes the tangents have (0 for one vehicle)"""
+        B, N = self.batch, self.n_nodes
+        tans, has_k = [], False
+        for i, (t, shape) in enumerate(zip((dx0, dyref, dyref_e, dw, dwe), ((13,), (N, 17), (13,), (17,), (13,)))):
+            if t is None:
+                tans.append(None)
+                continue
+            t = (t if torch.is_tensor(t) else torch.as_tensor(np.asarray(t, dtype=np.float64))).to(self.device, torch.float64)
+            if i >= 3 and t.dim() == len(shape):              # one weight direction shared by every vehicle
+                t = t.expand(B, *shape)
+            elif lead == 0:
+                t = t.unsqueeze(0)
+            extra = t.dim() - 1 - len(shape)                 # 1: a direction axis after the vehicle axis
+            if extra not in (0, 1) or t.shape[0] != B or tuple(t.shape[1 + extra:]) != shape:
+                raise ValueError(f"eval_jvp: tangent {i} has shape {tuple(t.shape)}, expected [B,(K,)]{list(shape)}")
+            has_k |= extra == 1
+            tans.append(t if extra else t.unsqueeze(1))
+        ks = {t.shape[1] for t in tans if t is not None}
+        if len(ks) > 1:
+            raise ValueError(f"eval_jvp: the tangents disagree on the number of directions, {sorted(ks)}")
+        K = ks.pop() if ks else 1
+        tans = [None if t is None else t.contiguous() for t in tans]
+        dx = torch.empty((B, K, N + 1, 13), dtype=torch.float64, device=self.device)
+        du = torch.empty((B, K, N, 4), dtype=torch.float64, device=self.device)
+        _capi.check(_capi.lib().qmpc_eval_jvp(self._h, K, *(_capi.ptr(t) for t in tans), _capi.ptr(dx), _capi.ptr(du),
+                                              self._s()))
+        return (dx, du) if has_k else (dx[:, 0], du[:, 0])
+
     def set_weights(self, w_diag=None, we_diag=None):
         """qmpc_set_weights: replace the stage weights diag(W) (17 entries) and/or the terminal weights diag(W_e) (13)
         for every later solve; None keeps that part.  numpy arrays or tensors.  The iterate and the warm-start active
@@ -221,8 +265,12 @@ class quad_optimizer:
         gradient is the one at that fixed linearisation.
         w_diag [17] / we_diag [13] (tensors, shared by every vehicle): the cost weights of this solve, set with
         set_weights before it (they stay on the handle); differentiable too, their gradient is the sum over vehicles
-        of eval_adjoint(weights=True)'s w_bar / we_bar.  None keeps the handle's weights, which count as constants."""
-        if iterate is not None and any(torch.is_tensor(t) and t.requires_grad for t in iterate):
+        of eval_adjoint(weights=True)'s w_bar / we_bar.  None keeps the handle's weights, which count as constants.
+        Forward mode too (torch.autograd.forward_ad, torch.func.jvp): the jvp is eval_jvp with the transposed mapping
+        (dyref = (dx_ref, du_ref), dyref_N = dx_ref[:, N-1], the weight tangents shared by every vehicle), under the
+        same conditions as the backward; it runs right after the forward."""
+        if iterate is not None and any(torch.is_tensor(t) and (t.requires_grad or fwAD.unpack_dual(t).tangent is not None)
+                                       for t in iterate):
             raise ValueError("differentiable_step: the iterate is the linearisation point and is not differentiated; "
                              "pass it detached")
         return _RTIStep.apply(self, x0, x_ref, u_ref, iterate, w_diag, we_diag)
@@ -314,12 +362,21 @@ class quad_optimizer:
                                              C.c_double(0.0 if odometry_dt is None else float(odometry_dt)), self._s()))
 
 
+def _plain(t):
+    """the tensor under torch.func's wrappers: torch.func.jvp hands a Function's jvp wrapped tangents, and the kernels
+    need their storage"""
+    t = t.detach()
+    while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        t = torch._C._functorch.get_unwrapped(t)
+    return t
+
+
 class _RTIStep(torch.autograd.Function):
     """quad_optimizer.differentiable_step: forward = one RTI solve, backward = qmpc_eval_adjoint (qmpc_eval_adjoint_weights
-    when the weights need a gradient) on that solve's tiles"""
+    when the weights need a gradient) on that solve's tiles, jvp = qmpc_eval_jvp with the transposed mapping"""
 
     @staticmethod
-    def forward(ctx, opt, x0, x_ref, u_ref, iterate, w_diag, we_diag):
+    def forward(opt, x0, x_ref, u_ref, iterate, w_diag, we_diag):
         B, N = opt.batch, opt.n_nodes
         if w_diag is not None or we_diag is not None:
             opt.set_weights(w_diag, we_diag)
@@ -328,21 +385,28 @@ class _RTIStep(torch.autograd.Function):
         if iterate is not None:
             opt.set_iterate(*iterate)
         x, u, _, _ = opt.run_optimization(x0.detach().to(opt.device, torch.float64).reshape(B, 13))
-        ctx.opt, ctx.epoch = opt, opt.sens_epoch()
-        ctx.like = [(t.shape, t.device, t.dtype) if torch.is_tensor(t) else None
-                    for t in (x0, x_ref, u_ref, iterate, w_diag, we_diag)]
-        ctx.set_materialize_grads(False)
         lead = x0.shape[:-1]
         return x.reshape(*lead, N + 1, 13), u.reshape(*lead, N, 4)
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        opt = inputs[0]
+        ctx.opt, ctx.epoch = opt, opt.sens_epoch()
+        ctx.like = [(t.shape, t.device, t.dtype) if torch.is_tensor(t) else None for t in inputs[1:]]
+        ctx.set_materialize_grads(False)
+
+    @staticmethod
+    def _check_epoch(ctx):
+        if ctx.opt.sens_epoch() != ctx.epoch:
+            raise RuntimeError("differentiable_step: the handle has solved again or had its active set changed since "
+                               "this step's forward; the stage tiles and active set its backward needs are gone")
 
     @staticmethod
     def backward(ctx, x_bar, u_bar):
         opt = ctx.opt
         if x_bar is None and u_bar is None:
             return None, None, None, None, None, None, None
-        if opt.sens_epoch() != ctx.epoch:
-            raise RuntimeError("differentiable_step: the handle has solved again or had its active set changed since "
-                               "this step's forward; the stage tiles and active set its backward needs are gone")
+        _RTIStep._check_epoch(ctx)
         weights = ctx.needs_input_grad[5] or ctx.needs_input_grad[6]
         out = opt._adjoint(x_bar, u_bar, weights)
         x0b, yb, yeb = out[:3]
@@ -352,3 +416,34 @@ class _RTIStep(torch.autograd.Function):
         like = lambda g, i: g.reshape(ctx.like[i][0]).to(ctx.like[i][1], ctx.like[i][2]) if ctx.needs_input_grad[i + 1] else None
         wb, web = (out[3].sum(0), out[4].sum(0)) if weights else (None, None)    # the weights are shared by the vehicles
         return None, like(x0b, 0), like(x_ref_bar, 1), like(yb[..., 13:], 2), None, like(wb, 4), like(web, 5)
+
+    @staticmethod
+    def jvp(ctx, _opt_t, x0_t, x_ref_t, u_ref_t, _iterate_t, w_t, we_t):
+        """the transpose of backward's mapping: dyref = (dx_ref, du_ref), dyref_e = dx_ref[:, N-1], the weight tangents
+        shared by every vehicle"""
+        opt = ctx.opt
+        B, N = opt.batch, opt.n_nodes
+        lead = ctx.like[0][0][:-1]
+        if x0_t is None and x_ref_t is None and u_ref_t is None and w_t is None and we_t is None:
+            z = lambda *shape: torch.zeros((*lead, *shape), dtype=torch.float64, device=opt.device)
+            return z(N + 1, 13), z(N, 4)
+        _RTIStep._check_epoch(ctx)
+        with torch._C._DisableFuncTorch():            # plain tensors for the kernel, as in forward
+            return _RTIStep._jvp_plain(opt, lead, *(None if t is None else _plain(t)
+                                                    for t in (x0_t, x_ref_t, u_ref_t, w_t, we_t)))
+
+    @staticmethod
+    def _jvp_plain(opt, lead, x0_t, x_ref_t, u_ref_t, w_t, we_t):
+        B, N = opt.batch, opt.n_nodes
+        f64 = lambda t, *shape: None if t is None else t.to(opt.device, torch.float64).reshape(*shape)
+        dx0 = f64(x0_t, B, 13)
+        dyref = dyref_e = None
+        if x_ref_t is not None or u_ref_t is not None:
+            dyref = torch.zeros((B, N, 17), dtype=torch.float64, device=opt.device)
+            if x_ref_t is not None:
+                dyref[..., :13] = f64(x_ref_t, B, N, 13)
+                dyref_e = dyref[:, N - 1, :13].contiguous()   # yref_e = x_ref[:, N-1] (set_reference_kernel)
+            if u_ref_t is not None:
+                dyref[..., 13:] = f64(u_ref_t, B, N, 4)
+        dx, du = opt._jvp(dx0, dyref, dyref_e, f64(w_t, 17), f64(we_t, 13))
+        return dx.reshape(*lead, N + 1, 13), du.reshape(*lead, N, 4)

@@ -1,5 +1,6 @@
 """Cost of qmpc_eval_sens_x0 (derivatives of the RTI step w.r.t. x0), of qmpc_eval_adjoint (its reverse mode, w.r.t. x0
-and the reference) and of qmpc_eval_adjoint_weights (also w.r.t. the cost weights) beside the solve they differentiate.
+and the reference), of qmpc_eval_adjoint_weights (also w.r.t. the cost weights) and of qmpc_eval_jvp (the forward mode
+w.r.t. all of them) beside the solve they differentiate.
 
 Workload: bench.py's random_smooth closed loop, B = 4096, N = 20, M = 20, fp64; 40 fused closed-loop steps first (the
 last 20 with qmpc_timing_* on, for the solve time), then 200 timed calls of each case with CUDA events around every call:
@@ -8,6 +9,9 @@ last 20 with qmpc_timing_* on, for the solve time), then 200 timed calls of each
   adjoint       qmpc_eval_adjoint with u_bar on stage 0 only (x_bar NULL), all three outputs
   adjoint_full  qmpc_eval_adjoint with every cotangent (x_bar and u_bar), all three outputs
   adjoint_weights  qmpc_eval_adjoint_weights with every cotangent, all five outputs
+  jvp_full      qmpc_eval_jvp, K = 1 direction with every tangent (dx0, dyref, dyref_e, dw, dwe), dx and du
+  jvp_x0_13     qmpc_eval_jvp, K = 13 unit directions of x0 (what eval_sens(N) with states returns), dx and du
+  jvp_weights_30  qmpc_eval_jvp, K = 30 unit directions of the cost weights (17 of w_diag, 13 of we_diag), dx and du
 Prints one JSON line and writes it to --out.  Needs a GPU.
 
     python scripts/bench_sens.py --out bench_outputs/sens.json
@@ -130,6 +134,34 @@ def main():
         ok = opt.solver_status()[0] == 0
         finite = all(bool(torch.isfinite(o[ok]).all()) for o in ((x0b, yb, yeb, wb, web) if weights else (x0b, yb, yeb)))
         out[name] = {"x_bar": xbp is not None, "u_bar": "stage 0" if name == "adjoint" else "all",
+                     "median_ms": float(np.median(t)), "p99_ms": float(np.percentile(t, 99)), "min_ms": float(t.min()),
+                     "vehicles_status_ok": int(ok.sum().item()), "finite_for_status_ok": finite}
+
+    # forward mode: the tangents are drawn once; the unit directions are what a Jacobian of the plan needs
+    f64 = dict(dtype=torch.float64, device=dev)
+    full = [torch.randn((B, 1) + sh, **f64, generator=g) for sh in ((13,), (N, 17), (13,), (17,), (13,))]
+    eye13 = torch.eye(13, **f64).expand(B, 13, 13).contiguous()
+    eye30 = torch.eye(30, **f64).expand(B, 30, 30)
+    wdirs = [None, None, None, eye30[..., :17].contiguous(), eye30[..., 17:].contiguous()]
+    jvp = {"jvp_full": (1, full), "jvp_x0_13": (13, [eye13, None, None, None, None]), "jvp_weights_30": (30, wdirs)}
+    for name, (K, tans) in jvp.items():
+        dxo = torch.empty((B, K, N + 1, 13), **f64)
+        duo = torch.empty((B, K, N, 4), **f64)
+        call = lambda: _capi.check(lib.qmpc_eval_jvp(opt._h, K, *(_capi.ptr(t) for t in tans), _capi.ptr(dxo),
+                                                     _capi.ptr(duo), s))
+        for _ in range(10):
+            call()
+        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.calls)]
+        for e0, e1 in ev:
+            e0.record()
+            call()
+            e1.record()
+        torch.cuda.synchronize()
+        t = np.array([e0.elapsed_time(e1) for e0, e1 in ev])
+        ok = opt.solver_status()[0] == 0
+        finite = bool(torch.isfinite(dxo[ok]).all()) and bool(torch.isfinite(duo[ok]).all())
+        out[name] = {"n_dir": K, "tangents": [n for n, tt in zip(("dx0", "dyref", "dyref_e", "dw", "dwe"), tans)
+                                              if tt is not None],
                      "median_ms": float(np.median(t)), "p99_ms": float(np.percentile(t, 99)), "min_ms": float(t.min()),
                      "vehicles_status_ok": int(ok.sum().item()), "finite_for_status_ok": finite}
     line = json.dumps(out)
